@@ -425,6 +425,8 @@ def ours(args):
         solve_s, wall = float(t[0]), float(t[1])
     per_step = solve_s / args.steps
     value = n_glob * iters / per_step
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, drv, driver, dist, rank, row_start, n_loc, n_glob)
     if os.environ.get("HDK_TIMELINE") == "1":             # diagnostics: per-operation times of one more solve, to stderr
         hdk.tune("timeline", 1)
         one_solve()
@@ -588,6 +590,49 @@ def companion_parity(hdk, driver, dist, cfg, rank, world):
     return out
 
 
+DUMP_SAMPLE = 1 << 20    # solution entries written by --dump-outputs (8 MB in float64)
+
+
+def dump_positions(n_glob):
+    """Global solution positions written by --dump-outputs: all of them up to DUMP_SAMPLE, else
+    DUMP_SAMPLE draws with a fixed seed, sorted and without repeats (the same for the same grid)."""
+    import numpy as np
+    if n_glob <= DUMP_SAMPLE:
+        return np.arange(n_glob)
+    return np.unique(np.random.default_rng(0).integers(0, n_glob, DUMP_SAMPLE))
+
+
+def gather_dump_sample(x_loc, row_start, n_glob, dist=None):
+    """The solution at dump_positions(n_glob), from each rank's slab x_loc (global rows row_start..);
+    collective at N > 1, where ranks hold consecutive slabs in rank order."""
+    import numpy as np
+    idx = dump_positions(n_glob)
+    mine = idx[(idx >= row_start) & (idx < row_start + len(x_loc))] - row_start
+    x = np.asarray(x_loc, dtype=np.float64)[mine]
+    if dist is not None:
+        parts = [None] * dist.get_world_size()
+        dist.all_gather_object(parts, x)
+        x = np.concatenate(parts)
+    return x
+
+
+def dump_outputs(outdir, drv, driver, dist, rank, row_start, n_loc, n_glob):
+    """What the last timed solve hands its caller, as float64 .npy files under `outdir` (rank 0):
+    solution.npy (at dump_positions), iterations.npy and final_rel_res_norm.npy (shape (1,)).
+    Collective at N > 1."""
+    import numpy as np
+    L = driver.api()
+    pv, it, rr = C.POINTER(C.c_double)(), C.c_int(), C.c_double()
+    driver._check(L.HYPREDRV_LinearSystemGetSolutionValues(drv._h, C.byref(pv)), "GetSolutionValues")
+    driver._check(L.HYPREDRV_LinearSolverGetNumIter(drv._h, C.byref(it)), "GetNumIter")
+    driver._check(L.HYPREDRV_LinearSolverGetFinalRelativeResidualNorm(drv._h, C.byref(rr)), "GetFinalRelRes")
+    x = gather_dump_sample(np.ctypeslib.as_array(pv, shape=(n_loc,)), row_start, n_glob, dist)
+    if rank == 0:
+        os.makedirs(outdir, exist_ok=True)
+        np.save(os.path.join(outdir, "solution.npy"), x)
+        np.save(os.path.join(outdir, "iterations.npy"), np.array([it.value], dtype=np.float64))
+        np.save(os.path.join(outdir, "final_rel_res_norm.npy"), np.array([rr.value], dtype=np.float64))
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -598,7 +643,14 @@ def main():
                     help="BASELINE.json configuration (default: the 256^3 headline)")
     ap.add_argument("--n", type=int, default=0, help="development override: cube edge instead of the config's")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed solve returned (solution, "
+                         "iterations, final relative residual norm) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     args.cfg = CONFIGS[args.config]
     if args.n:                                    # development override of the cube edge (both arms)

@@ -195,6 +195,42 @@ def test_ij_shim_containers():
     assert L.HYPRE_IJVectorDestroy(v) == 0 and L.HYPRE_IJMatrixDestroy(A) == 0
 
 
+def test_mpi_shim_cartesian_and_point_to_point(monkeypatch):
+    """include/mpi.h without an MPI library: one process is exact (every Cartesian neighbour is
+    MPI_PROC_NULL, point-to-point calls to it succeed and move nothing); with several processes of
+    the launcher environment the Cartesian calls follow MPI's row-major rank order, and a
+    point-to-point call to a real peer fails instead of returning wrong data."""
+    L = hdk.lib()
+    WORLD, PROC_NULL, INT = 1, -2, 1
+    I3 = C.c_int * 3
+    monkeypatch.delenv("WORLD_SIZE", raising=False)
+    monkeypatch.delenv("RANK", raising=False)
+    cart, src, dst, req, coords = C.c_int(), C.c_int(), C.c_int(), C.c_int(7), I3()
+    assert L.MPI_Cart_create(WORLD, 3, I3(1, 1, 1), I3(0, 0, 0), 0, C.byref(cart)) == 0
+    for d in range(3):
+        assert L.MPI_Cart_shift(cart, d, 1, C.byref(src), C.byref(dst)) == 0
+        assert (src.value, dst.value) == (PROC_NULL, PROC_NULL)
+    buf = (C.c_int * 4)(1, 2, 3, 4)
+    assert L.MPI_Isend(buf, 4, INT, PROC_NULL, 0, cart, C.byref(req)) == 0 and req.value == 0
+    assert L.MPI_Irecv(buf, 4, INT, PROC_NULL, 0, cart, C.byref(req)) == 0 and list(buf) == [1, 2, 3, 4]
+    assert L.MPI_Waitall(0, None, None) == 0
+    assert L.MPI_Comm_free(C.byref(cart)) == 0 and cart.value == 0
+    # rank 1 of a 1 x 1 x 2 grid
+    monkeypatch.setenv("WORLD_SIZE", "2")
+    monkeypatch.setenv("RANK", "1")
+    assert L.MPI_Cart_create(WORLD, 3, I3(1, 1, 3), I3(0, 0, 0), 0, C.byref(cart)) != 0   # 3 processes on 2
+    assert L.MPI_Cart_create(WORLD, 3, I3(1, 1, 2), I3(0, 0, 0), 0, C.byref(cart)) == 0
+    assert L.MPI_Cart_coords(cart, 1, 3, coords) == 0 and list(coords) == [0, 0, 1]
+    r = C.c_int()
+    assert L.MPI_Cart_rank(cart, I3(0, 0, 0), C.byref(r)) == 0 and r.value == 0
+    assert L.MPI_Cart_shift(cart, 2, 1, C.byref(src), C.byref(dst)) == 0 and (src.value, dst.value) == (0, PROC_NULL)
+    assert L.MPI_Cart_shift(cart, 0, 1, C.byref(src), C.byref(dst)) == 0 and (src.value, dst.value) == (PROC_NULL, PROC_NULL)
+    assert L.MPI_Isend(buf, 4, INT, 0, 0, cart, C.byref(req)) != 0
+    assert L.MPI_Irecv(buf, 4, INT, 0, 0, cart, C.byref(req)) != 0
+    assert L.MPI_Isend(buf, 4, INT, PROC_NULL, 0, cart, C.byref(req)) == 0
+    assert L.MPI_Comm_free(C.byref(cart)) == 0
+
+
 def test_options_dict_to_yaml():
     y = driver.normalize_options({"general": {"statistics": False}, "solver": {"pcg": {"max_iter": 10}},
                                   "preconditioner": {"amg": {"print_level": 0}}})

@@ -267,3 +267,41 @@ def test_initial_guess_previous_across_two_systems(gpu):
         res = hd.solve(A, b, options={"general": {"statistics": False}, "linear_system": {"init_guess_mode": mode},
                                       "solver": {"pcg": {"relative_tol": 1e-9, "max_iter": 100}}, "preconditioner": "amg"})
         assert res.converged and np.linalg.norm(b - A @ res.x) <= 1e-9 * np.linalg.norm(b) * 1.0001
+
+
+def test_bench_dump_outputs(gpu, tmp_path):
+    """`bench.py --dump-outputs DIR` writes what the last of `--steps` timed solves returned: the
+    solution at the seeded sample of positions (a 104^3 grid has more than DUMP_SAMPLE rows), its
+    iteration count and final relative residual norm.  `--steps` sets how many solves are timed:
+    three steps launch three times the kernels of one."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+    n = 104
+
+    def run(steps):
+        out = tmp_path / f"steps{steps}"
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", str(steps),
+                            "--warmup", "1", "--n", str(n), "--no-cpu-baseline", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads(r.stdout.strip().splitlines()[-1])
+        return line, [np.load(out / f"{k}.npy") for k in ("solution", "iterations", "final_rel_res_norm")]
+
+    line1, (x1, it1, rr1) = run(1)
+    line3, (x3, it3, rr3) = run(3)
+    assert line1["gpu_launches"] > 0 and line3["gpu_launches"] == 3 * line1["gpu_launches"]
+    idx = bench.dump_positions(n ** 3)
+    assert idx.size < n ** 3
+    for x, it, rr, line in ((x1, it1, rr1, line1), (x3, it3, rr3, line3)):
+        assert x.dtype == it.dtype == rr.dtype == np.float64 and x.shape == idx.shape and it.shape == rr.shape == (1,)
+        assert int(it[0]) == line["iterations"] and 0 < rr[0] < 1e-6
+    A, b = O.gen("lap7", n, n, n)
+    xo, io = O.pcg(A, b, M=O.Hierarchy(A, O.default_params(True)), rel_tol=1e-6, max_iter=100)
+    assert int(it1[0]) == int(it3[0]) == io["iters"]
+    for x in (x1, x3):
+        assert np.linalg.norm(x - xo[idx]) <= 1e-8 * np.linalg.norm(xo[idx])

@@ -1,13 +1,17 @@
-"""The reference's OWN callers, compiled unmodified against include/ + libHYPREDRV.so (recipe
-oracle/build_ref_callers.sh, run by __graft_entry__.build() where /root/reference exists; the
-binaries travel to the GPU box under oracle/_ref/):
-  * examples/src/C_laplacian/laplacian.c  -- `laplacian -n 10 10 10`: the STATISTICS table must
-    have the layout of the reference's golden output (examples/refOutput/laplacian.txt,
-    transcribed into tests/golden/laplacian_layout.json) with the same initial residual norm;
-    the iteration count is the GPU-default chain's (PMIS + l1-Jacobi), checked against the oracle;
-    also as two ranks (`-P 1 1 2`, communicator from the launcher environment).
-  * tests/test_setmatrix_from_csr.c       -- the reference's unit test of the CSR ingest path runs
-    green (its own assertions: error bits, known answers, offset slabs)."""
+"""C callers of the HYPREDRV_* API, built by __graft_entry__.build() from tests/callers/ against
+include/ + libHYPREDRV.so only, as an application links it:
+  * laplacian.c -- the 7-point problem of hypredrive's C_laplacian example on a Cartesian process
+    grid (MPI_Cart_* of the include/mpi.h shim), assembled through the HYPRE_IJ interface and
+    solved five times.  `laplacian -n 10 10 10`: the STATISTICS table the library prints must have
+    the layout of the reference's golden output (examples/refOutput/laplacian.txt, transcribed into
+    tests/golden/laplacian_layout.json) with the same initial residual norm; the iteration count is
+    the GPU-default chain's (PMIS + l1-Jacobi), checked against the oracle; also as two ranks
+    (`-P 1 1 2`, communicator from the launcher environment).  The banner lines before the table
+    are the program's own (its command line, and the process grid as the Cartesian communicator
+    reports it).
+  * csr_ingest.c -- unit test of the CSR ingest path: error bits through the error-module entry
+    points, HYPRE_Int overflow, empty rows, ownership of CSR input and of a caller's IJ objects
+    across matrix replacements, known answers, offset indptr slabs."""
 import json
 import os
 import re
@@ -19,17 +23,17 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REFBIN = os.path.join(ROOT, "oracle", "_ref")
+REFBIN = os.path.join(ROOT, "build", "callers")
 
 
 def _need(name):
     p = os.path.join(REFBIN, name)
     if not os.path.exists(p):
-        pytest.fail(f"{p} missing: run __graft_entry__.build() where /root/reference is present")
+        pytest.fail(f"{p} missing: run __graft_entry__.build()")
     return p
 
 
-def test_reference_laplacian_driver_runs_against_this_library(gpu):
+def test_laplacian_example_runs_against_this_library(gpu):
     from oracle import oracle as O
     exe = _need("laplacian")
     r = subprocess.run([exe, "-n", "10", "10", "10"], capture_output=True, text=True, timeout=300, cwd=ROOT)
@@ -55,14 +59,14 @@ def test_reference_laplacian_driver_runs_against_this_library(gpu):
         assert float(cells[5]) < 1e-6 and int(cells[6]) == info["iters"]
 
 
-def test_reference_unit_test_of_the_csr_ingest_path(gpu):
-    exe = _need("test_setmatrix_from_csr")
+def test_csr_ingest_unit_test(gpu):
+    exe = _need("csr_ingest")
     r = subprocess.run([exe], capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
 
 
-def test_reference_laplacian_driver_as_two_ranks(gpu, tmp_path):
-    """The same unmodified example as TWO processes (its own `-P 1 1 2` z-split and MPI calls on the
+def test_laplacian_example_as_two_ranks(gpu, tmp_path):
+    """The same example as TWO processes (`-P 1 1 2`: a 1 x 1 x 2 Cartesian communicator of the
     `include/mpi.h` shim): the communicator comes from the launcher environment
     (`hdk_comm_init_from_env`, rank 0 publishes the NCCL id in a file), the hierarchy is set up
     row-distributed, and the printed iteration count / residual are the oracle's for the whole grid."""

@@ -106,3 +106,45 @@ def test_slab_ranges_cover_everything():
         assert rng[0][0] == 0 and rng[-1][1] == n - 1
         assert all(rng[r][1] + 1 == rng[r + 1][0] for r in range(w - 1))
         assert all(e >= s for s, e in rng)
+
+
+def _dump_worker(rank, world, port, n_glob, out):
+    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    import bench
+    x = np.random.default_rng(5).standard_normal(n_glob)
+    cuts = [n_glob * r // world for r in range(world + 1)]             # uneven consecutive slabs
+    got = bench.gather_dump_sample(x[cuts[rank]:cuts[rank + 1]], cuts[rank], n_glob, dist)
+    if rank == 0:
+        out.put(bool(np.array_equal(got, x[bench.dump_positions(n_glob)])))
+    dist.barrier()
+    dist.destroy_process_group()
+
+
+def test_bench_dump_sample_gathered_over_two_ranks_gloo():
+    """bench.py --dump-outputs at N > 1: each rank contributes its slab's entries of the seeded
+    sample, and rank 0 receives them in global order."""
+    n_glob = 3_000_001
+    ctx = mp.get_context("spawn")
+    out = ctx.Queue()
+    procs = [ctx.Process(target=_dump_worker, args=(r, 2, 29735, n_glob, out)) for r in range(2)]
+    for p in procs:
+        p.start()
+    assert out.get(timeout=180) is True
+    for p in procs:
+        p.join(timeout=60)
+        assert p.exitcode == 0
+
+
+def test_bench_dump_positions(monkeypatch):
+    """Whole solution up to DUMP_SAMPLE entries; beyond, a seeded sample: sorted, unique, in range,
+    the same on every call, and at most DUMP_SAMPLE positions."""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 1000)
+    assert np.array_equal(bench.dump_positions(1000), np.arange(1000))
+    idx = bench.dump_positions(50_000)
+    assert 900 < idx.size <= 1000 and idx[0] >= 0 and idx[-1] < 50_000 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(idx, bench.dump_positions(50_000))
+    x = np.arange(50_000) * 0.5
+    assert np.array_equal(bench.gather_dump_sample(x, 0, 50_000), x[idx])
+    assert np.array_equal(bench.gather_dump_sample(x[20_000:], 20_000, 50_000), x[idx[idx >= 20_000]])
