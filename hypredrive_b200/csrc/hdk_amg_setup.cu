@@ -835,7 +835,11 @@ __global__ void __launch_bounds__(32 * IW_WARPS) k_interp_warp(const int *arp, c
    __syncwarp();
    int  nC = 0, nins = 0;
    bool overflow = false;
-   // ---- discovery of C-hat_i; strong F neighbours are tagged with idx = -2
+   // ---- discovery of C-hat_i; strong F neighbours are tagged with idx = -2.  The row overflows once
+   // |C-hat| > IW_LIST or the inserts (C-hat plus strong F neighbours) exceed IW_INS; the count is
+   // checked after every insert (of at most 32 keys), so the table never holds more than IW_INS + 32
+   // keys and never fills: in a full open-addressing table wt_find_or_insert would probe forever.
+   constexpr int IW_INS = (IW_CAP * 3) / 4;
    for (int jj = srp[i]; jj < srp[i + 1] && !overflow; jj++)
    {
       const int i1 = scol[jj], c1 = cf[i1];
@@ -850,12 +854,14 @@ __global__ void __launch_bounds__(32 * IW_WARPS) k_interp_warp(const int *arp, c
             if (nC >= IW_LIST) overflow = true;
             else if (lane == 0) { idx[h] = nC; lc[nC] = i1; lv[nC] = 0.0; }
             nC++; nins++;
+            if (nins > IW_INS) overflow = true;
          }
       }
       else if (c1 != SF_PT)
       {
          if (lane == 0) { bool nw; int h = wt_find_or_insert(keys, IW_CAP, i1, nw); idx[h] = -2; }
          nins++;
+         if (nins > IW_INS) overflow = true;
          __syncwarp();
          for (int base = srp[i1]; base < srp[i1 + 1] && !overflow; base += 32)
          {
@@ -867,7 +873,7 @@ __global__ void __launch_bounds__(32 * IW_WARPS) k_interp_warp(const int *arp, c
             if (act) h = wt_find_or_insert(keys, IW_CAP, k1, isnew);
             const unsigned nm = __ballot_sync(FULL, act && isnew);
             const int      add = __popc(nm);
-            if (nC + add > IW_LIST || nins + add > (IW_CAP * 3) / 4) overflow = true;
+            if (nC + add > IW_LIST || nins + add > IW_INS) overflow = true;
             else if (act && isnew) { int s = nC + __popc(nm & LT); idx[h] = s; lc[s] = k1; lv[s] = 0.0; }
             nC += add; nins += add;
             __syncwarp();
@@ -1871,7 +1877,7 @@ static int build_lower(const DevCSR &A, DevCSR &L)
 }
 
 // =====================================================================================
-// coarsest level: dense inverse by Gauss-Jordan with partial pivoting, one CTA
+// coarsest level: dense inverse by Gauss-Jordan with partial pivoting (one CTA up to GJ_ONE_CTA rows)
 // =====================================================================================
 __global__ void k_dense_fill(const int *rp, const int *col, const double *val, int n, double *M /* n x 2n */)
 {
@@ -1934,17 +1940,95 @@ __global__ void __launch_bounds__(1024) k_gauss_jordan(double *M, int n, double 
    for (int idx = tid; idx < n * n; idx += nt) { int r = idx / n, j = idx - r * n; inv[idx] = M[(size_t)r * w + n + j]; }
 }
 
+// The same elimination for coarsest operators of more than GJ_ONE_CTA rows, two launches per pivot
+// step over the whole grid: k_gj_pivot (one CTA) picks, swaps and scales the pivot row and saves
+// the multipliers of column k in f; k_gj_eliminate updates every other row.  Each entry sees the
+// same operations in the same order as in k_gauss_jordan.  Left of column k the pivot row is zero.
+constexpr int GJ_ONE_CTA = 1024;
+__global__ void __launch_bounds__(1024) k_gj_pivot(double *M, int n, int k, double *f)
+{
+   __shared__ double sval[32];
+   __shared__ int    sidx[32];
+   __shared__ int    piv;
+   __shared__ double pivval;
+   const int tid = threadIdx.x, nt = blockDim.x, w = 2 * n;
+   double best = -1.0; int bi = k;
+   for (int r = k + tid; r < n; r += nt) { double v = fabs(M[(size_t)r * w + k]); if (v > best) { best = v; bi = r; } }
+   for (int o = 16; o > 0; o >>= 1)
+   {
+      double ov = __shfl_down_sync(0xffffffffu, best, o); int oi = __shfl_down_sync(0xffffffffu, bi, o);
+      if (ov > best || (ov == best && oi < bi)) { best = ov; bi = oi; }
+   }
+   if ((tid & 31) == 0) { sval[tid >> 5] = best; sidx[tid >> 5] = bi; }
+   __syncthreads();
+   if (tid == 0)
+   {
+      double b = sval[0]; int i2 = sidx[0];
+      for (int q = 1; q < (nt + 31) / 32; q++) if (sval[q] > b || (sval[q] == b && sidx[q] < i2)) { b = sval[q]; i2 = sidx[q]; }
+      piv = i2; pivval = M[(size_t)i2 * w + k];
+   }
+   __syncthreads();
+   const int    pr = piv;
+   const double pv = pivval;
+   if (pv != 0.0)
+   {
+      if (pr != k)
+         for (int j = tid; j < w; j += nt) { double t = M[(size_t)k * w + j]; M[(size_t)k * w + j] = M[(size_t)pr * w + j]; M[(size_t)pr * w + j] = t; }
+      __syncthreads();
+      for (int j = tid; j < w; j += nt) M[(size_t)k * w + j] /= pv;
+   }
+   // a zero pivot column leaves the step out: no multipliers
+   for (int r = tid; r < n; r += nt) f[r] = (pv != 0.0 && r != k) ? M[(size_t)r * w + k] : 0.0;
+}
+
+__global__ void k_gj_eliminate(double *M, int n, int k, const double *f)
+{
+   const int    r = blockIdx.y, w = 2 * n;
+   const double fr = f[r];
+   if (fr == 0.0) return; // (also the pivot row)
+   for (int j = k + blockIdx.x * blockDim.x + threadIdx.x; j < w; j += gridDim.x * blockDim.x)
+   {
+      if (j == k) M[(size_t)r * w + k] = 0.0;
+      else M[(size_t)r * w + j] -= fr * M[(size_t)k * w + j];
+   }
+}
+
+__global__ void k_gj_extract(const double *M, int n, double *inv)
+{
+   const int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+   if (idx >= (int64_t)n * n) return;
+   const int64_t r = idx / n, j = idx - r * n;
+   inv[idx] = M[r * 2 * n + n + j];
+}
+
 static int build_dense_inverse(const DevCSR &A, double **inv)
 {
    int     n = A.nrows;
    double *M;
    HDK_TRY(dalloc(&M, (size_t)n * 2 * n + 8));
-   HDK_TRY(dalloc(inv, (size_t)n * n + 8));
+   if (int rc = dalloc(inv, (size_t)n * n + 8)) { dfree(M); return rc; }
    HDK_CUDA(cudaMemsetAsync(M, 0, sizeof(double) * ((size_t)n * 2 * n), g.stream));
    k_dense_fill<<<cdiv(n, 128), 128, 0, g.stream>>>(A.rowptr, A.col, A.val, n, M);
    HDK_LAUNCH_CHECK();
-   k_gauss_jordan<<<1, 1024, 0, g.stream>>>(M, n, *inv);
-   HDK_LAUNCH_CHECK();
+   if (n <= GJ_ONE_CTA)
+   {
+      k_gauss_jordan<<<1, 1024, 0, g.stream>>>(M, n, *inv);
+      HDK_LAUNCH_CHECK();
+   }
+   else
+   {
+      double *f;
+      if (int rc = dalloc(&f, (size_t)n + 8)) { dfree(M); return rc; }
+      for (int k = 0; k < n; k++)
+      {
+         k_gj_pivot<<<1, 1024, 0, g.stream>>>(M, n, k, f);
+         k_gj_eliminate<<<dim3(cdiv(2 * n - k, 256), n), 256, 0, g.stream>>>(M, n, k, f);
+      }
+      HDK_LAUNCH_CHECK();
+      k_gj_extract<<<(unsigned)(((int64_t)n * n + 255) / 256), 256, 0, g.stream>>>(M, n, *inv);
+      HDK_LAUNCH_CHECK();
+      dfree(f);
+   }
    dfree(M);
    return HDK_OK;
 }
@@ -2139,7 +2223,9 @@ int setup_serial(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk_amg_s **out
    {
       AmgLevel &Lc = M->lev[(size_t)M->nlev - 1];
       bool      want_ge = (prm->relax_coarse == 9 || prm->relax_coarse == 99 || prm->relax_coarse == 19);
-      if (want_ge && Lc.n <= 1024 && Lc.n > 0 && Lc.A->offd.nnz == 0)
+      // hypre_GaussElimSetup builds the dense coarse matrix whatever its size; both this library and
+      // the CPU oracle cap it at n^2 < 2e8 (1.6 GB, about 14 000 rows) and relax above that
+      if (want_ge && (double)Lc.n * Lc.n < 2.0e8 && Lc.n > 0 && Lc.A->offd.nnz == 0)
       {
          rc = build_dense_inverse(Lc.A->diag, &M->ge_inv);
          M->ge_n = Lc.n;

@@ -9,7 +9,7 @@
 
 namespace hdk {
 
-// u = Ainv f  (n <= 1024): one warp per row of the dense inverse
+// u = Ainv f: one warp per row of the dense inverse (any n; size_t row offsets)
 __global__ void __launch_bounds__(256) k_dense_apply(const double *__restrict__ Ainv, const double *__restrict__ f,
                                                      double *__restrict__ u, int n)
 {

@@ -659,7 +659,8 @@ oamg *oamg_setup(const ocsr *Ain, const oamg_params *prm)
       h->t[l]  = (double *)calloc((size_t)n + 1, sizeof(double));
       h->t2[l] = (double *)calloc((size_t)n + 1, sizeof(double));
    }
-   /* coarsest level: dense copy for Gaussian elimination (hypre_GaussElimSetup) */
+   /* coarsest level: dense copy for Gaussian elimination (hypre_GaussElimSetup, which has no size
+    * limit; the n^2 < 2e8 cap bounds the copy to 1.6 GB and is the device's limit too) */
    if (prm->relax_coarse == 9 || prm->relax_coarse == 99 || h->nlev == 1)
    {
       ocsr *Ac = h->A[h->nlev - 1];

@@ -12,6 +12,7 @@ import os
 import sys
 
 import numpy as np
+import scipy.sparse as sp
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -47,16 +48,31 @@ def main():
     hdk.check(hdk.lib().hdk_comm_init(rank, world, bytes(uid.tolist())))
 
     kind = sys.argv[1] if len(sys.argv) > 1 else "lap7"
-    nx, ny, nzl = (int(v) for v in (sys.argv[2:5] if len(sys.argv) > 4 else (12, 11, 6)))
-    nz = nzl * world
-    code, c, solver, tol = {"lap7": (7, (1.0, 1.0, 1.0), "pcg", 1e-6), "lap27": (27, (1.0, 1.0, 0.01), "pcg", 1e-6),
-                            "convdif": (107, (1e-3, 1.0, 0.1), "gmres", 1e-8)}[kind]
-    n_tot = nx * ny * nz
+    amg_kw = {}
+    if kind == "npz":
+        # a general matrix and right-hand side written by the parent: npz <file> (indptr, indices,
+        # data, b; optional max_levels), every rank passes its slab of rows through the CSR API
+        sysdat = np.load(sys.argv[2])
+        A_ip, A_cj, A_va, b_all = sysdat["indptr"], sysdat["indices"], sysdat["data"], sysdat["b"]
+        if "max_levels" in sysdat:
+            amg_kw["max_levels"] = int(sysdat["max_levels"])
+        n_tot = b_all.size
+        solver, tol = "pcg", 1e-8
+        grid = f"n={n_tot}"
+    else:
+        nx, ny, nzl = (int(v) for v in (sys.argv[2:5] if len(sys.argv) > 4 else (12, 11, 6)))
+        nz = nzl * world
+        code, c, solver, tol = {"lap7": (7, (1.0, 1.0, 1.0), "pcg", 1e-6), "lap27": (27, (1.0, 1.0, 0.01), "pcg", 1e-6),
+                                "convdif": (107, (1e-3, 1.0, 0.1), "gmres", 1e-8)}[kind]
+        n_tot = nx * ny * nz
+        grid = f"grid={nx}x{ny}x{nz}"
     if os.environ.get("MPCHECK_RAGGED") == "1":
         # uneven slabs that cut through grid planes: rank r owns rows [cuts[r], cuts[r+1])
         w = np.array([1.0 + 0.7 * ((r * 37) % 5) for r in range(world)])
         cuts = np.concatenate([[0], np.floor(np.cumsum(w) / w.sum() * n_tot).astype(np.int64)])
         cuts[-1] = n_tot
+    elif kind == "npz":
+        cuts = np.arange(world + 1, dtype=np.int64) * n_tot // world
     else:
         cuts = np.arange(world + 1, dtype=np.int64) * (nx * ny * nzl)
     rs, re = int(cuts[rank]), int(cuts[rank + 1]) - 1
@@ -64,11 +80,16 @@ def main():
     if check_hier:
         hdk.tune("amg_keep_debug", 1)
     opts = {"general": {"statistics": False}, "solver": {solver: {"relative_tol": tol, "max_iter": 100}},
-            "preconditioner": "amg"}
+            "preconditioner": {"amg": {"coarsening": amg_kw}} if amg_kw else "amg"}
     L = driver.api()
     hier = None
     with driver.HypreDrive(options=opts) as drv:
-        drv.set_stencil(code, nx, ny, nz, c, rs, re)
+        if kind == "npz":
+            lo, hi = int(A_ip[rs]), int(A_ip[re + 1])
+            drv.set_matrix_from_csr(A_ip[rs:re + 2] - lo, A_cj[lo:hi], A_va[lo:hi], row_start=rs, row_end=re)
+            drv.set_rhs(b_all[rs:re + 1])
+        else:
+            drv.set_stencil(code, nx, ny, nz, c, rs, re)
         driver._check(L.HYPREDRV_LinearSystemSetInitialGuess(drv._h, None), "SetInitialGuess")
         driver._check(L.HYPREDRV_LinearSystemResetInitialGuess(drv._h), "ResetInitialGuess")
         driver._check(L.HYPREDRV_LinearSolverCreate(drv._h), "LinearSolverCreate")
@@ -116,8 +137,11 @@ def main():
     if rank == 0:
         from oracle import oracle as O
         x = torch.cat(xs).numpy()
-        A, b = O.gen(kind, nx, ny, nz, c=c)
-        H = O.Hierarchy(A, O.default_params(True))
+        if kind == "npz":
+            A, b = sp.csr_matrix((A_va, A_cj, A_ip), shape=(n_tot, n_tot)), b_all
+        else:
+            A, b = O.gen(kind, nx, ny, nz, c=c)
+        H = O.Hierarchy(A, O.default_params(True, **amg_kw))
         xr, ir = (O.pcg if solver == "pcg" else O.gmres)(A, b, M=H, rel_tol=tol, max_iter=100)
         rel = np.linalg.norm(x - xr) / np.linalg.norm(xr)
         res = np.linalg.norm(b - A @ x) / np.linalg.norm(b)
@@ -126,7 +150,7 @@ def main():
         if check_hier:
             hok, hmsg = compare_hierarchy(hiers, H)
             ok = ok and hok
-        print(f"MPCHECK kind={kind} world={world} grid={nx}x{ny}x{nz} iters={iters} oracle_iters={ir['iters']} "
+        print(f"MPCHECK kind={kind} world={world} {grid} levels={H.sizes()} iters={iters} oracle_iters={ir['iters']} "
               f"rel_diff={rel:.2e} true_res={res:.2e} {hmsg} ok={ok}", flush=True)
     flag = torch.tensor([1 if ok else 0])
     dist.broadcast(flag, 0)

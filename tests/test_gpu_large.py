@@ -1,6 +1,7 @@
 """GPU parity at sizes where the production code paths are the ones that run (>= 10^6 rows):
-natural sliced-ELL selection (>= 200 000 rows), the warp-per-row setup kernels with their
-fall-backs, chunked scratch, every level of a 7-8 level hierarchy.  The CUDA hierarchy is
+natural sliced-ELL selection (>= 200 000 rows), the warp-per-row setup kernels, every level of a
+7-8 level hierarchy.  (The setup's scratch stays below one chunk at these sizes; the fall-back
+paths for long rows are reached by tests/test_gpu_unstructured.py.)  The CUDA hierarchy is
 compared with an oracle run of the same problem level by level -- sizes, C/F splitting,
 interpolation and Galerkin operators bit for bit (pattern, storage order and values) -- and the
 Krylov solve by iteration count (north star: +-1), solution difference <= 1e-8 and true residual."""

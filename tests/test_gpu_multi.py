@@ -114,3 +114,48 @@ def _row_distributed_case(world, kind, dims, rep, ragged, extra):
     r = _run(world, [kind, *dims], env)
     assert r.returncode == 0, _digest(r)
     assert "ok=True" in r.stdout and "hier=bit-identical" in r.stdout, _digest(r)
+
+
+def _npz_system(path, name, max_levels=None):
+    """One of tests/amg_paths.py's cases in hypre's storage (diagonal first, as the oracle orders
+    it), with a random right-hand side, written for the ranks of mp_gpu_check.py."""
+    import numpy as np
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import amg_paths as AP
+    A = AP.CASES[name][0]().tocsr()
+    for i in range(A.shape[0]):                  # ocsr_diag_first: swap the diagonal into first place
+        b, e = A.indptr[i], A.indptr[i + 1]
+        k = b + int(np.nonzero(A.indices[b:e] == i)[0][0])
+        A.indices[[b, k]], A.data[[b, k]] = A.indices[[k, b]], A.data[[k, b]]
+    extra = {} if max_levels is None else {"max_levels": np.int64(max_levels)}
+    np.savez(path, indptr=A.indptr.astype(np.int64), indices=A.indices.astype(np.int64), data=A.data,
+             b=AP.rhs(A.shape[0]), **extra)
+
+
+@pytest.mark.parametrize("world,ragged", [(2, "0"), (3, "1")])
+@pytest.mark.parametrize("mode", ["share", "sell-fused"])
+def test_heavy_tailed_graph_on_several_ranks(gpu, tmp_path, world, ragged, mode):
+    """The heavy-tailed graph (hubs with hundreds of scattered columns) through the CSR API on 2
+    ranks and on 3 ragged slabs: the exported rows are spread over every slab, the setup's long-row
+    fallbacks run on distributed levels.  Hierarchy bit-identical to the oracle's, solve parity."""
+    path = str(tmp_path / "system.npz")
+    _npz_system(path, "heavy_tailed")
+    env = {"HDK_REPLICATE_ROWS": "2000", "MPCHECK_RAGGED": ragged, "MPCHECK_HIER": "1"}
+    if mode == "share":
+        env["HDK_SHARE_MIN_ROWS"] = "0"
+    else:
+        env.update(HDK_SELL_MIN_ROWS="0", HDK_SELL_MIN_ROWS_DIST="0")
+    r = _run(world, ["npz", path], env)
+    assert r.returncode == 0, _digest(r)
+    assert "ok=True" in r.stdout and "hier=bit-identical" in r.stdout, _digest(r)
+
+
+def test_coarse_direct_solve_above_one_cta_on_two_ranks(gpu, tmp_path):
+    """max_levels 2 on a 12 000-row graph: a replicated coarsest level of more than 1024 rows, whose
+    dense inverse every rank builds with the grid-wide Gauss-Jordan elimination."""
+    path = str(tmp_path / "system.npz")
+    _npz_system(path, "two_levels", max_levels=2)
+    r = _run(2, ["npz", path], {"HDK_REPLICATE_ROWS": "2000", "MPCHECK_RAGGED": "1", "MPCHECK_HIER": "1",
+                               "HDK_SHARE_MIN_ROWS": "0"})
+    assert r.returncode == 0, _digest(r)
+    assert "ok=True" in r.stdout and "hier=bit-identical" in r.stdout, _digest(r)
