@@ -14,6 +14,7 @@ struct AmgLevel
    int       *cf = nullptr;
    int       *f2c = nullptr; // exclusive scan of (cf > 0), n+1 entries (kept for the N > 1 slicing)
    double    *measure = nullptr;
+   int       *dof = nullptr;     // function labels of the rows (systems AMG, num_functions > 1)
    double    *l1_down = nullptr, *l1_up = nullptr; // smoother diagonals (may alias)
    double    *u = nullptr, *f = nullptr, *t = nullptr;
    double    *gs1 = nullptr, *gs2 = nullptr; // two-stage GS: correction vectors of the inner steps
@@ -57,12 +58,15 @@ struct hdk_amg_s
 // pieces of the serial setup (hdk_amg_setup.cu) that the distributed driver (hdk_amg_dist.cu) reuses
 extern "C" {
 int finalize_levels(hdk_amg_s *M, const hdk_amg_params *prm, int64_t live_max_rows);
-int setup_serial(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk_amg_s **out, bool keep_f2c, int64_t live_max_rows);
+// dof0_d: device labels of the rows of A0 (systems AMG); nullptr: prm->dof_func or interleaved labels
+int setup_serial(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk_amg_s **out, bool keep_f2c, int64_t live_max_rows,
+                 const int *dof0_d = nullptr);
 int setup_distributed_rows(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk_amg_s **out); // hdk_amg_dist.cu
 }
 
 namespace hdk {
-int build_strength_csr(const DevCSR &D, const int *orp, const double *ov, double theta, double mrs, DevCSR &S);
+int build_strength_csr(const DevCSR &D, const int *orp, const double *ov, double theta, double mrs, DevCSR &S,
+                       const int *dof = nullptr);
 int pmis_count_cols(const DevCSR &S, int row0, int n, int *cnt);
 int pmis_measure(const int *cnt, int n, int seed, int64_t goff, double *measure);
 int pmis_init(const DevCSR &S, int row0, int n, int *cf, double *measure);
@@ -70,7 +74,7 @@ int pmis_mark(int n, int *cf, const double *measure);
 int pmis_elim(const DevCSR &S, int row0, int n, int *cf, const double *measure);
 int pmis_set(const DevCSR &S, int row0, int n, int *cf, double *measure, int *remaining);
 int build_interp(const DevCSR &A, const DevCSR &S, int *cf, const int *f2c, int nc, int max_elmts_in, double trunc_factor,
-                 DevCSR &P, int row_lo, int row_hi);
+                 DevCSR &P, int row_lo, int row_hi, const int *dof = nullptr);
 int build_rap(const DevCSR &R, const DevCSR &A, const DevCSR &P, DevCSR &C, int row_lo, int row_hi);
 int csr_transpose(const DevCSR &A, DevCSR &T);
 hdk_csr_s *wrap_local(DevCSR &D, int64_t grows);

@@ -214,14 +214,19 @@ __device__ __forceinline__ int wt_find_or_insert(int *keys, int cap, int key, bo
 // =====================================================================================
 struct RowS { double diag, thr; bool weak_all; };
 
+// SYS (num_functions > 1, unknown approach): row_scale and row_sum run over the couplings to the
+// row's own function only (dof = function labels); the caller guarantees orp == nullptr
+template <bool SYS = false>
 __device__ __forceinline__ RowS row_strength(const int *rp, const double *val, const int *orp, const double *oval,
-                                             int i, double theta, double mrs)
+                                             int i, double theta, double mrs, const int *col = nullptr, const int *dof = nullptr)
 {
    RowS   r;
    int    b = rp[i], e = rp[i + 1];
    double diag = val[b], row_scale = 0.0, row_sum = diag;
+   const int di = SYS ? dof[i] : 0;
    for (int k = b + 1; k < e; k++)
    {
+      if (SYS && dof[col[k]] != di) continue;
       double v = val[k];
       if (diag < 0) row_scale = row_scale > v ? row_scale : v;
       else row_scale = row_scale < v ? row_scale : v;
@@ -241,9 +246,9 @@ __device__ __forceinline__ RowS row_strength(const int *rp, const double *val, c
    return r;
 }
 
-template <bool FILL>
+template <bool FILL, bool SYS = false>
 __global__ void k_strength(const int *rp, const int *col, const double *val, const int *orp, const double *oval,
-                           int n, double theta, double mrs, int *cnt, const int *srp, int *scol)
+                           int n, double theta, double mrs, int *cnt, const int *srp, int *scol, const int *dof = nullptr)
 {
    int i = blockIdx.x * blockDim.x + threadIdx.x;
    if (i > n) return;
@@ -252,25 +257,29 @@ __global__ void k_strength(const int *rp, const int *col, const double *val, con
    int p = FILL ? srp[i] : 0;
    if (e > b)
    {
-      RowS r = row_strength(rp, val, orp, oval, i, theta, mrs);
+      RowS r = row_strength<SYS>(rp, val, orp, oval, i, theta, mrs, col, dof);
       if (!r.weak_all)
          for (int k = b + 1; k < e; k++)
          {
             double v      = val[k];
             bool   strong = (r.diag < 0) ? !(v <= r.thr) : !(v >= r.thr);
+            if (SYS) strong = strong && dof[col[k]] == dof[i];
             if (strong) { if (FILL) scol[p++] = col[k]; else c++; }
          }
    }
    if (!FILL) cnt[i] = c;
 }
 
-int build_strength_csr(const DevCSR &D, const int *orp, const double *ov, double theta, double mrs, DevCSR &S)
+int build_strength_csr(const DevCSR &D, const int *orp, const double *ov, double theta, double mrs, DevCSR &S, const int *dof)
 {
    int n = D.nrows;
+   // systems AMG runs on one rank or on the replicated global matrix: there is no off-diagonal block
+   if (dof && orp) return set_error(HDK_ERR_UNSUPPORTED, "systems AMG strength: the matrix has an off-processor block");
    int *cnt, *srp;
    HDK_TRY(dalloc(&cnt, (size_t)n + 1));
    HDK_TRY(dalloc(&srp, (size_t)n + 1));
-   k_strength<false><<<cdiv(n + 1, 256), 256, 0, g.stream>>>(D.rowptr, D.col, D.val, orp, ov, n, theta, mrs, cnt, nullptr, nullptr);
+   if (dof) k_strength<false, true><<<cdiv(n + 1, 256), 256, 0, g.stream>>>(D.rowptr, D.col, D.val, orp, ov, n, theta, mrs, cnt, nullptr, nullptr, dof);
+   else k_strength<false><<<cdiv(n + 1, 256), 256, 0, g.stream>>>(D.rowptr, D.col, D.val, orp, ov, n, theta, mrs, cnt, nullptr, nullptr);
    HDK_LAUNCH_CHECK();
    HDK_TRY(exclusive_scan_int(cnt, srp, n + 1));
    int nnzS = 0;
@@ -280,16 +289,17 @@ int build_strength_csr(const DevCSR &D, const int *orp, const double *ov, double
    S = DevCSR();
    S.nrows = n; S.ncols = n; S.nnz = nnzS; S.rowptr = srp; S.owns = true;
    HDK_TRY(dalloc(&S.col, (size_t)nnzS + 8));
-   k_strength<true><<<cdiv(n + 1, 256), 256, 0, g.stream>>>(D.rowptr, D.col, D.val, orp, ov, n, theta, mrs, nullptr, srp, S.col);
+   if (dof) k_strength<true, true><<<cdiv(n + 1, 256), 256, 0, g.stream>>>(D.rowptr, D.col, D.val, orp, ov, n, theta, mrs, nullptr, srp, S.col, dof);
+   else k_strength<true><<<cdiv(n + 1, 256), 256, 0, g.stream>>>(D.rowptr, D.col, D.val, orp, ov, n, theta, mrs, nullptr, srp, S.col);
    HDK_LAUNCH_CHECK();
    return HDK_OK;
 }
 
-static int build_strength(const hdk_csr_s &A, double theta, double mrs, DevCSR &S)
+static int build_strength(const hdk_csr_s &A, double theta, double mrs, DevCSR &S, const int *dof = nullptr)
 {
    const int    *orp = A.offd.nnz > 0 ? A.offd.rowptr : nullptr;
    const double *ov  = A.offd.nnz > 0 ? A.offd.val : nullptr;
-   return build_strength_csr(A.diag, orp, ov, theta, mrs, S);
+   return build_strength_csr(A.diag, orp, ov, theta, mrs, S, dof);
 }
 
 // =====================================================================================
@@ -468,6 +478,19 @@ int pmis_set(const DevCSR &S, int row0, int n, int *cf, double *measure, int *re
    return HDK_OK;
 }
 
+// systems AMG: hypre's default labels (global row modulo num_functions), and the labels of the
+// C points carried to the coarse level in coarse order (hypre_BoomerAMGCoarseParms)
+__global__ void k_dof_interleaved(int n, int64_t goff, int nf, int *dof)
+{
+   int i = blockIdx.x * blockDim.x + threadIdx.x;
+   if (i < n) dof[i] = (int)((goff + i) % nf);
+}
+__global__ void k_dof_coarse(const int *cf, const int *f2c, const int *dof, int n, int *dof_c)
+{
+   int i = blockIdx.x * blockDim.x + threadIdx.x;
+   if (i < n && cf[i] > 0) dof_c[f2c[i]] = dof[i];
+}
+
 __global__ void k_cf_flag(const int *cf, int n, int *flag)
 {
    int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -577,10 +600,13 @@ __device__ void qsort2abs_dev(int *v, double *w, int n, int keep)
    }
 }
 
+// SYS (num_functions > 1): a weak coupling to another function (dof = function labels) is dropped
+// instead of being lumped into the diagonal; the same flag in k_interp_small and k_interp_warp
+template <bool SYS = false>
 __global__ void k_interp_fill(const int *arp, const int *acol, const double *aval, const int *srp, const int *scol,
                               const int *cf, const int *f2c, int row0, int row1, const int *cnt,
                               const int64_t *hoff, int2 *htab, const int64_t *loff, int *lcol, double *lval,
-                              int max_elmts, const int *prp, int *pcol, double *pval, const int *slow)
+                              int max_elmts, const int *prp, int *pcol, double *pval, const int *slow, const int *dof = nullptr)
 {
    int i = row0 + blockIdx.x * blockDim.x + threadIdx.x;
    if (i >= row1 || !slow[i]) return;
@@ -644,7 +670,7 @@ __global__ void k_interp_fill(const int *arp, const int *acol, const double *ava
          }
          else diagonal = __dadd_rn(diagonal, a);
       }
-      else if (cf[i1] != SF_PT) diagonal = __dadd_rn(diagonal, a);
+      else if (cf[i1] != SF_PT && (!SYS || dof[i1] == dof[i])) diagonal = __dadd_rn(diagonal, a);
    }
    if (diagonal != 0.0)
    {
@@ -683,9 +709,11 @@ __device__ __forceinline__ int is_find(const int *key, int n, int k)
       if (key[j] == k) return j;
    return -1;
 }
+template <bool SYS = false>
 __global__ void __launch_bounds__(128) k_interp_small(const int *arp, const int *acol, const double *aval, const int *srp,
                                                       const int *scol, const int *cf, const int *f2c, int row_lo, int row_hi,
-                                                      int max_elmts, int *cnt, int *rowlen, int *slow, int *scol_out, double *sval_out)
+                                                      int max_elmts, int *cnt, int *rowlen, int *slow, int *scol_out, double *sval_out,
+                                                      const int *dof = nullptr)
 {
    const int i = row_lo + blockIdx.x * blockDim.x + threadIdx.x;
    if (i >= row_hi) return;
@@ -753,7 +781,7 @@ __global__ void __launch_bounds__(128) k_interp_small(const int *arp, const int 
          }
          else diagonal = __dadd_rn(diagonal, a);
       }
-      else if (cf[i1] != SF_PT) diagonal = __dadd_rn(diagonal, a);
+      else if (cf[i1] != SF_PT && (!SYS || dof[i1] == dof[i])) diagonal = __dadd_rn(diagonal, a);
    }
    if (diagonal != 0.0)
    {
@@ -801,12 +829,12 @@ __device__ __forceinline__ int wt_find(const int *keys, const int *idx, int cap,
 // STAGE (single-pass interpolation, max_elmts > 0): discovery AND weights in one launch; the truncated
 // row (at most max_elmts entries) goes to slot i * max_elmts of a staging buffer and cnt / rowlen / slow
 // are set like the counting pass does, so no row is traversed twice.
-template <bool FILL, bool STAGE = false>
+template <bool FILL, bool STAGE = false, bool SYS = false>
 __global__ void __launch_bounds__(32 * IW_WARPS) k_interp_warp(const int *arp, const int *acol, const double *aval,
                                                                const int *srp, const int *scol, const int *cf,
                                                                const int *f2c, int n, int max_elmts, int *cnt, int *rowlen,
                                                                int *slow, const int *prp, int *pcol, double *pval, int force_slow,
-                                                               int row_lo)
+                                                               int row_lo, const int *dof = nullptr)
 {
    __shared__ int    s_keys[IW_WARPS][IW_CAP];
    __shared__ int    s_idx[IW_WARPS][IW_CAP];
@@ -897,6 +925,7 @@ __global__ void __launch_bounds__(32 * IW_WARPS) k_interp_warp(const int *arp, c
    // shuffles, so the sequential loop has no chain of dependent global loads.
    const int rs = arp[i], re = arp[i + 1];
    double    diagonal = aval[rs];
+   const int di = SYS ? dof[i] : 0;
    for (int cb = rs + 1; cb < re; cb += 32)
    {
       const int    jl = cb + lane;
@@ -915,7 +944,7 @@ __global__ void __launch_bounds__(32 * IW_WARPS) k_interp_warp(const int *arp, c
             p_sgn = aval[d1] < 0 ? -1.0 : 1.0;
             p_b1  = d1 + 1;
          }
-         else if (p_m < 0) p_cf = cf[p_i1];
+         else if (p_m < 0) p_cf = (SYS && dof[p_i1] != di) ? SF_PT : cf[p_i1]; // (SYS: another function's weak coupling is dropped)
       }
       const int nchunk = (re - cb) < 32 ? (re - cb) : 32;
       for (int t = 0; t < nchunk; t++)
@@ -1114,8 +1143,9 @@ static int interp_truncate(DevCSR &P, double trunc_factor, int max_elmts)
 }
 
 // rows [row_lo, row_hi) only (row_lo < 0: all rows, or this rank's share of a work-shared global level)
+// dof != nullptr: systems AMG, the SYS variants of the three interpolation kernels
 int build_interp(const DevCSR &A, const DevCSR &S, int *cf, const int *f2c, int nc, int max_elmts_in, double trunc_factor,
-                 DevCSR &P, int row_lo, int row_hi)
+                 DevCSR &P, int row_lo, int row_hi, const int *dof)
 {
    // with a truncation factor the rows are built complete and truncated by the post-pass
    const int max_elmts = (trunc_factor > 0.0) ? 0 : max_elmts_in;
@@ -1159,10 +1189,16 @@ int build_interp(const DevCSR &A, const DevCSR &S, int *cf, const int *f2c, int 
       HDK_TRY(dalloc(&stg_val, (size_t)n * max_elmts + 8));
       if (force_slow) // short rows: one thread per row with thread-local tables
       {
-         if (hi > lo)
+         if (hi > lo && dof)
+            k_interp_small<true><<<cdiv(hi - lo, 128), 128, 0, g.stream>>>(A.rowptr, A.col, A.val, S.rowptr, S.col, cf, f2c, lo, hi, max_elmts,
+                                                                           cnt, rowlen, slow, stg_col, stg_val, dof);
+         else if (hi > lo)
             k_interp_small<<<cdiv(hi - lo, 128), 128, 0, g.stream>>>(A.rowptr, A.col, A.val, S.rowptr, S.col, cf, f2c, lo, hi, max_elmts,
                                                                      cnt, rowlen, slow, stg_col, stg_val);
       }
+      else if (dof)
+         k_interp_warp<true, true, true><<<cdiv(hi - lo, IW_WARPS), 32 * IW_WARPS, 0, g.stream>>>(A.rowptr, A.col, A.val, S.rowptr, S.col, cf, f2c, hi,
+                                                                                                  max_elmts, cnt, rowlen, slow, nullptr, stg_col, stg_val, 0, lo, dof);
       else
          k_interp_warp<true, true><<<cdiv(hi - lo, IW_WARPS), 32 * IW_WARPS, 0, g.stream>>>(A.rowptr, A.col, A.val, S.rowptr, S.col, cf, f2c, hi,
                                                                                             max_elmts, cnt, rowlen, slow, nullptr, stg_col, stg_val, 0, lo);
@@ -1218,6 +1254,12 @@ int build_interp(const DevCSR &A, const DevCSR &S, int *cf, const int *f2c, int 
       HDK_LAUNCH_CHECK();
       dfree(stg_col); dfree(stg_val);
    }
+   else if (dof)
+   {
+      k_interp_warp<true, false, true><<<cdiv(hi - lo, IW_WARPS), 32 * IW_WARPS, 0, g.stream>>>(A.rowptr, A.col, A.val, S.rowptr, S.col, cf, f2c, hi,
+                                                                                               max_elmts, cnt, rowlen, slow, prp, P.col, P.val, force_slow, lo, dof);
+      HDK_LAUNCH_CHECK();
+   }
    else
    {
       k_interp_warp<true><<<cdiv(hi - lo, IW_WARPS), 32 * IW_WARPS, 0, g.stream>>>(A.rowptr, A.col, A.val, S.rowptr, S.col, cf, f2c, hi,
@@ -1252,8 +1294,12 @@ int build_interp(const DevCSR &A, const DevCSR &S, int *cf, const int *f2c, int 
          int r0 = bounds[c], r1 = bounds[c + 1];
          if (r1 <= r0) continue;
          HDK_CUDA(cudaMemsetAsync(htab, 0xFF, sizeof(int2) * ((size_t)maxsz + 4), g.stream));
-         k_interp_fill<<<cdiv(r1 - r0, 128), 128, 0, g.stream>>>(A.rowptr, A.col, A.val, S.rowptr, S.col, cf, f2c, r0, r1,
-                                                                cnt, off, htab, loff, lcol, lval, max_elmts, prp, P.col, P.val, slow);
+         if (dof)
+            k_interp_fill<true><<<cdiv(r1 - r0, 128), 128, 0, g.stream>>>(A.rowptr, A.col, A.val, S.rowptr, S.col, cf, f2c, r0, r1,
+                                                                          cnt, off, htab, loff, lcol, lval, max_elmts, prp, P.col, P.val, slow, dof);
+         else
+            k_interp_fill<<<cdiv(r1 - r0, 128), 128, 0, g.stream>>>(A.rowptr, A.col, A.val, S.rowptr, S.col, cf, f2c, r0, r1,
+                                                                   cnt, off, htab, loff, lcol, lval, max_elmts, prp, P.col, P.val, slow);
          HDK_LAUNCH_CHECK();
       }
       dfree(htab); dfree(lcol); dfree(lval);
@@ -2068,6 +2114,7 @@ void hdk_amg_default_params(hdk_amg_params *p)
    p->sweeps_down = p->sweeps_up = p->sweeps_coarse = 1;
    p->relax_weight = p->outer_weight = 1.0;
    p->rand_seed = 2747; p->keep_transpose = 1; p->print_level = 0;
+   p->num_functions = 1; p->dof_func = NULL;
 }
 
 int hdk_amg_destroy(hdk_amg *M)
@@ -2080,7 +2127,7 @@ int hdk_amg_destroy(hdk_amg *M)
          if (L.owns_A) destroy_local(L.A);
          destroy_local(L.P); destroy_local(L.R);
          csr_free(L.S); csr_free(L.L);
-         dfree(L.cf); dfree(L.measure); dfree(L.f2c);
+         dfree(L.cf); dfree(L.measure); dfree(L.f2c); dfree(L.dof);
          if (L.l1_up != L.l1_down) dfree(L.l1_up);
          dfree(L.l1_down);
          dfree(L.u); dfree(L.f); dfree(L.t); dfree(L.gs1); dfree(L.gs2);
@@ -2140,10 +2187,11 @@ int finalize_levels(hdk_amg_s *M, const hdk_amg_params *prm, int64_t live_max_ro
 // live_max_rows >= 0: the hierarchy is the global one of a multi-rank setup; levels with more
 // rows are only sliced into slabs afterwards, so they get no SpMV analysis and no solve data
 int setup_serial(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk_amg_s **out, bool keep_f2c,
-                 int64_t live_max_rows)
+                 int64_t live_max_rows, const int *dof0_d)
 {
    hdk_amg_s *M = new hdk_amg_s();
    M->prm       = *prm;
+   M->prm.dof_func = nullptr; // the caller's array is read here only
    M->keep_f2c  = keep_f2c;
    M->keep_debug = tune_amg_keep_debug();
    int rc       = HDK_OK;
@@ -2154,13 +2202,40 @@ int setup_serial(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk_amg_s **out
    int  level = 0;
    bool more  = prm->max_levels > 1;
    double nnz0 = (double)A0->diag.nnz + A0->offd.nnz, nnz_sum = nnz0;
+   const bool sys = prm->num_functions > 1;
+   if (sys)
+   {
+      const int n0 = M->lev[0].n;
+      int      *d  = nullptr;
+      rc = dalloc(&d, (size_t)n0 + 1);
+      M->lev[0].dof = d;
+      if (rc == HDK_OK && dof0_d)
+         rc = cudaMemcpyAsync(d, dof0_d, sizeof(int) * (size_t)n0, cudaMemcpyDeviceToDevice, g.stream) == cudaSuccess
+                 ? HDK_OK : set_error(HDK_ERR_CUDA, "copy of the function labels failed");
+      else if (rc == HDK_OK && prm->dof_func)
+      {
+         for (int i = 0; i < n0 && rc == HDK_OK; i++)
+            if (prm->dof_func[i] < 0 || prm->dof_func[i] >= prm->num_functions)
+               rc = set_error(HDK_ERR_INVALID, "dof_func[%d] = %d is outside [0, num_functions = %d)", i, (int)prm->dof_func[i], prm->num_functions);
+         if (rc == HDK_OK)
+            rc = cudaMemcpyAsync(d, prm->dof_func, sizeof(int) * (size_t)n0, cudaMemcpyHostToDevice, g.stream) == cudaSuccess
+                    ? HDK_OK : set_error(HDK_ERR_CUDA, "copy of the function labels failed");
+         if (rc == HDK_OK) rc = cudaStreamSynchronize(g.stream) == cudaSuccess ? HDK_OK : set_error(HDK_ERR_CUDA, "copy of the function labels failed");
+      }
+      else if (rc == HDK_OK && n0 > 0)
+      {
+         k_dof_interleaved<<<cdiv(n0, 256), 256, 0, g.stream>>>(n0, A0->row_start, prm->num_functions, d);
+         g.launches++;
+      }
+   }
+   int *dof_c = nullptr; // labels of the next level until that level exists
    while (more && rc == HDK_OK)
    {
       AmgLevel        &L = M->lev[(size_t)level];
       const hdk_csr_s &A = *L.A;
       int              n = L.n;
       stage_mark(nullptr, level);
-      if ((rc = build_strength(A, prm->strong_th, prm->max_row_sum, L.S))) break;
+      if ((rc = build_strength(A, prm->strong_th, prm->max_row_sum, L.S, sys ? L.dof : nullptr))) break;
       stage_mark("strength", level);
       if ((rc = dalloc(&L.cf, (size_t)n + 1))) break;
       double *meas, *keep = nullptr;
@@ -2184,8 +2259,13 @@ int setup_serial(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk_amg_s **out
       dfree(flag);
       if (nc == 0 || nc == n || nc < prm->min_coarse_size) { dfree(f2c); break; }
       DevCSR P, R, C;
-      rc = build_interp(A.diag, L.S, L.cf, f2c, nc, prm->max_nnz_row, prm->trunc_factor, P, -1, -1);
+      rc = build_interp(A.diag, L.S, L.cf, f2c, nc, prm->max_nnz_row, prm->trunc_factor, P, -1, -1, sys ? L.dof : nullptr);
       stage_mark("interp", level);
+      if (rc == HDK_OK && sys && (rc = dalloc(&dof_c, (size_t)nc + 1)) == HDK_OK)
+      {
+         k_dof_coarse<<<cdiv(n, 256), 256, 0, g.stream>>>(L.cf, f2c, L.dof, n, dof_c);
+         g.launches++;
+      }
       if (keep_f2c) L.f2c = f2c; else dfree(f2c);
       if (rc) break;
       if ((rc = csr_transpose(P, R))) break;
@@ -2208,11 +2288,12 @@ int setup_serial(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk_amg_s **out
       L.R = wrap_local(R, nc);
       M->lev.emplace_back();
       AmgLevel &N = M->lev.back();
-      N.A = wrap_local(C, nc); N.owns_A = true; N.n = nc;
+      N.A = wrap_local(C, nc); N.owns_A = true; N.n = nc; N.dof = dof_c; dof_c = nullptr;
       level++;
       if (level == prm->max_levels - 1 || nc <= prm->max_coarse_size) more = false;
       if (!M->keep_debug) csr_free(M->lev[(size_t)level - 1].S);
    }
+   dfree(dof_c);
    if (rc == HDK_OK)
    {
       M->nlev = level + 1;
@@ -2322,18 +2403,44 @@ static int setup_distributed(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk
       HDK_TRY(bcast_bytes(gcj + koff[(size_t)r], sizeof(int64_t) * (size_t)nnz_all[(size_t)r], r));
       HDK_TRY(bcast_bytes(gva + koff[(size_t)r], sizeof(double) * (size_t)nnz_all[(size_t)r], r));
    }
+   // systems AMG with explicit labels: the labels of every rank's rows, gathered like the matrix slabs
+   // (interleaved labels follow from the global row inside setup_serial)
+   int *gdof = nullptr;
+   if (prm->num_functions > 1 && prm->dof_func)
+   {
+      const int64_t nme = rows_all[(size_t)me];
+      int64_t       bad = -1;
+      for (int64_t i = 0; i < nme && bad < 0; i++)
+         if (prm->dof_func[i] < 0 || prm->dof_func[i] >= prm->num_functions) bad = i;
+      std::vector<int64_t> bad_all;
+      HDK_TRY(allgather_i64_host(bad, bad_all));
+      for (int r = 0; r < R; r++)
+         if (bad_all[(size_t)r] >= 0)
+         {
+            dfree(gip); dfree(gcj); dfree(gva);
+            return set_error(HDK_ERR_INVALID, "rank %d: dof_func[%lld] is outside [0, num_functions = %d)", r,
+                             (long long)bad_all[(size_t)r], prm->num_functions);
+         }
+      HDK_TRY(dalloc(&gdof, (size_t)N + 1));
+      HDK_CUDA(cudaMemcpyAsync(gdof + roff[(size_t)me], prm->dof_func, sizeof(int) * (size_t)nme, cudaMemcpyHostToDevice, g.stream));
+      for (int r = 0; r < R; r++) HDK_TRY(bcast_bytes(gdof + roff[(size_t)r], sizeof(int) * (size_t)rows_all[(size_t)r], r));
+   }
+   hdk_amg_params gprm = *prm;
+   gprm.dof_func = nullptr; // prm->dof_func holds this rank's rows only
    const int64_t rep_rows = tune_replicate_rows();
    hdk_csr_s *G = nullptr;
    int rc = parcsr_build(0, N - 1, 0, N - 1, N, N, true, false, false, gip, gcj, gva, &G, N <= rep_rows);
    dfree(gip); dfree(gcj); dfree(gva);
-   if (rc) return rc;
+   if (rc) { dfree(gdof); return rc; }
    // 3. the global hierarchy (serial algorithm, identical on every rank)
    stage_mark("gather A", -2);
    hdk_amg_s *Mg = nullptr;
    g_share = !(getenv("HDK_SETUP_SHARE") && atoi(getenv("HDK_SETUP_SHARE")) == 0);
    if (getenv("HDK_SHARE_MIN_ROWS")) g_share_min_rows = atoi(getenv("HDK_SHARE_MIN_ROWS"));
-   rc = setup_serial(G, prm, &Mg, true, rep_rows);
+   rc = setup_serial(G, &gprm, &Mg, true, rep_rows, gdof);
    g_share = false;
+   HDK_CUDA(cudaStreamSynchronize(g.stream));
+   dfree(gdof);
    if (rc) { destroy_local(G); return rc; }
    Mg->lev[0].owns_A = true; // G belongs to the global hierarchy
    stage_mark("global setup", -2);
@@ -2391,6 +2498,11 @@ static int setup_distributed(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk
          if ((rc = slice_rows(Lg.P->diag, (int)fs, (int)fe, 0, nc - 1, nf, nc, false, false, &L.P))) break;
       }
       if ((rc = slice_rows(Lg.R->diag, (int)cs, (int)ce, fs, fe - 1, nc, nf, false, true, &L.R))) break;
+      if (Lg.dof) // this rank's labels (introspection: hdk_amg_get_dof_func)
+      {
+         if ((rc = dalloc(&L.dof, (size_t)L.n + 1))) break;
+         HDK_CUDA(cudaMemcpyAsync(L.dof, Lg.dof + fs, sizeof(int) * (size_t)L.n, cudaMemcpyDeviceToDevice, g.stream));
+      }
    }
    stage_mark("slice", -2);
    if (rc == HDK_OK)
@@ -2424,6 +2536,7 @@ static int setup_distributed(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk
          destroy_local(Lg.R); Lg.R = nullptr;
          csr_free(Lg.S); csr_free(Lg.L);
          dfree(Lg.cf); Lg.cf = nullptr; dfree(Lg.measure); Lg.measure = nullptr; dfree(Lg.f2c); Lg.f2c = nullptr;
+         dfree(Lg.dof); Lg.dof = nullptr;
          if (Lg.l1_up != Lg.l1_down) dfree(Lg.l1_up);
          dfree(Lg.l1_down); Lg.l1_down = Lg.l1_up = nullptr;
          dfree(Lg.u); dfree(Lg.f); dfree(Lg.t); Lg.u = Lg.f = Lg.t = nullptr;
@@ -2442,13 +2555,16 @@ int hdk_amg_setup(const hdk_csr *A0, const hdk_amg_params *prm, hdk_amg **out)
    if (!A0 || !prm || !out) return set_error(HDK_ERR_INVALID, "hdk_amg_setup: null argument");
    if (prm->interp_type != 6) return set_error(HDK_ERR_UNSUPPORTED, "interpolation type %d: only extended+i (6) has a device kernel", prm->interp_type);
    if (prm->trunc_factor < 0.0 || prm->trunc_factor >= 1.0) return set_error(HDK_ERR_INVALID, "interpolation trunc_factor must be in [0, 1)");
+   if (prm->num_functions < 1) return set_error(HDK_ERR_INVALID, "num_functions must be at least 1 (got %d)", prm->num_functions);
    g_timing = getenv("HDK_SETUP_TIMING") && atoi(getenv("HDK_SETUP_TIMING")) == 1;
    // row-distributed setup (hdk_amg_dist.cu); HDK_SETUP_REPLICATED=1 selects the round-1 scheme that
    // rebuilds the global hierarchy on every rank (kept for comparison)
    const bool replicated = getenv("HDK_SETUP_REPLICATED") && atoi(getenv("HDK_SETUP_REPLICATED")) == 1;
    const bool force_dist = getenv("HDK_SETUP_DIST_FORCE") && atoi(getenv("HDK_SETUP_DIST_FORCE")) == 1;
-   if (g.nranks > 1 && replicated) return setup_distributed(A0, prm, out);
-   if (g.nranks > 1 || (force_dist && A0->orig_indptr)) return setup_distributed_rows(A0, prm, out);
+   // systems AMG has no row-distributed setup yet: N > 1 rebuilds the global hierarchy on every rank
+   const bool sys = prm->num_functions > 1;
+   if (g.nranks > 1 && (replicated || sys)) return setup_distributed(A0, prm, out);
+   if (!sys && (g.nranks > 1 || (force_dist && A0->orig_indptr))) return setup_distributed_rows(A0, prm, out);
    return setup_serial(A0, prm, out, false, -1);
 }
 
@@ -2506,6 +2622,13 @@ int hdk_amg_get_cf(const hdk_amg *M, int level, int32_t *cf_h)
    M = resolve_level(M, level);
    if (!M || level < 0 || level >= M->nlev) return set_error(HDK_ERR_INVALID, "level out of range");
    return get_level_array(M, level, M->lev[(size_t)level].cf, sizeof(int) * (size_t)M->lev[(size_t)level].n, cf_h);
+}
+int hdk_amg_get_dof_func(const hdk_amg *M, int level, int32_t *dof_h)
+{
+   M = resolve_level(M, level);
+   if (!M || level < 0 || level >= M->nlev) return set_error(HDK_ERR_INVALID, "level out of range");
+   if (!M->lev[(size_t)level].dof) return set_error(HDK_ERR_INVALID, "no function labels: the hierarchy was built with num_functions = 1");
+   return get_level_array(M, level, M->lev[(size_t)level].dof, sizeof(int) * (size_t)M->lev[(size_t)level].n, dof_h);
 }
 int hdk_amg_get_measure(const hdk_amg *M, int level, double *m_h)
 {

@@ -784,6 +784,15 @@ uint32_t HYPREDRV_PreconCreate(HYPREDRV_t h)
    return hd_err_get();
 }
 
+uint32_t HYPREDRV_PreconGetDeviceParams(HYPREDRV_t h, void *params)
+{
+   CHECK_ARGS(h);
+   if (!params) return fail(HYPREDRV_ERROR_INVALID_VAL, "%s", "null parameter block");
+   if (hd_amg_check(&h->args->amg)) return hd_err_get();
+   hd_amg_to_hdk(&h->args->amg, (hdk_amg_params *)params);
+   return hd_err_get();
+}
+
 static uint32_t do_precon_setup(HYPREDRV_t h)
 {
    if (!h->A) return fail(HYPREDRV_ERROR_INVALID_VAL, "%s", "the matrix must be set before the preconditioner setup");
@@ -794,6 +803,7 @@ static uint32_t do_precon_setup(HYPREDRV_t h)
    if (h->args->precon_method == HD_PRECON_AMG)
    {
       hdk_amg_params p;
+      if (hd_amg_check(&h->args->amg)) return hd_err_get();
       hd_amg_to_hdk(&h->args->amg, &p);
       if (p.coarsen_type != 8)
       {

@@ -611,4 +611,31 @@ void hd_amg_to_hdk(const hd_amg_args *a, hdk_amg_params *p)
    p->sweeps_coarse = a->coarse_sweeps > -1 ? a->coarse_sweeps : a->num_sweeps;
    p->relax_weight = a->weight; p->outer_weight = a->outer_weight;
    p->keep_transpose = a->keep_transpose; p->print_level = a->print_level;
+   p->num_functions = a->num_functions;
+}
+
+/* systems AMG (num_functions > 1) runs hypre's unknown approach only: the nodal approach and
+ * filter_functions would otherwise be ignored silently, so they are rejected */
+int hd_amg_check(const hd_amg_args *a)
+{
+   int bad = 0;
+   if (a->num_functions < 1)
+   {
+      hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+      hd_err_msg("amg:coarsening:num_functions must be at least 1 (got %d)", a->num_functions);
+      bad = 1;
+   }
+   if (a->num_functions > 1 && a->nodal)
+   {
+      hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+      hd_err_msg("amg:coarsening:nodal is not supported with num_functions = %d: only the unknown approach (nodal: 0) has a device setup", a->num_functions);
+      bad = 1;
+   }
+   if (a->num_functions > 1 && a->filter_functions)
+   {
+      hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+      hd_err_msg("amg:coarsening:filter_functions is not supported with num_functions = %d", a->num_functions);
+      bad = 1;
+   }
+   return bad;
 }

@@ -129,6 +129,7 @@ int  hd_args_apply_precon_preset(hd_args *a, const char *preset);
 int  hd_args_apply_solver_preset(hd_args *a, const char *preset);
 int  hd_preset_register(int kind, const char *name, const char *text, const char *help);
 void hd_amg_to_hdk(const hd_amg_args *a, hdk_amg_params *p);
+int  hd_amg_check(const hd_amg_args *a); /* 1 (error bit and message set): an option combination without a device path */
 /* 1 if the preconditioner must be rebuilt for the 0-based linear system `ls_id` */
 int  hd_reuse_should_rebuild(const hd_reuse_args *r, int ls_id);
 

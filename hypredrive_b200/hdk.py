@@ -26,7 +26,8 @@ class AmgParams(C.Structure):
                 ("relax_down", C.c_int), ("relax_up", C.c_int), ("relax_coarse", C.c_int),
                 ("sweeps_down", C.c_int), ("sweeps_up", C.c_int), ("sweeps_coarse", C.c_int),
                 ("relax_weight", C.c_double), ("outer_weight", C.c_double), ("rand_seed", C.c_int),
-                ("keep_transpose", C.c_int), ("print_level", C.c_int)]
+                ("keep_transpose", C.c_int), ("print_level", C.c_int),
+                ("num_functions", C.c_int), ("dof_func", C.POINTER(C.c_int32))]
 
 
 class Krylov(C.Structure):
@@ -82,6 +83,7 @@ def lib():
         L.hdk_amg_get_matrix.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
         L.hdk_amg_get_cf.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.hdk_amg_get_measure.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
+        L.hdk_amg_get_dof_func.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.hdk_amg_get_l1.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.hdk_pcg.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Krylov)]
         L.hdk_gmres.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Krylov)]
@@ -233,11 +235,16 @@ def amg_params(**kw) -> AmgParams:
 class DAmg:
     """Device BoomerAMG hierarchy."""
 
-    def __init__(self, A: DCsr, params: AmgParams | None = None):
+    def __init__(self, A: DCsr, params: AmgParams | None = None, dof_func=None):
+        """dof_func: this rank's row labels for systems AMG (params.num_functions > 1); None: interleaved."""
         self.params = params if params is not None else amg_params()
         self.h = C.c_void_p()
         self.A = A
+        if dof_func is not None:
+            dof = np.ascontiguousarray(dof_func, dtype=np.int32)
+            self.params.dof_func = dof.ctypes.data_as(C.POINTER(C.c_int32))
         check(lib().hdk_amg_setup(A.h, C.byref(self.params), C.byref(self.h)))
+        self.params.dof_func = None   # read during the setup only
 
     @property
     def nlev(self):
@@ -273,6 +280,12 @@ class DAmg:
     def cf(self, l):
         out = np.empty(self.level_info(l)["rows"], dtype=np.int32)
         check(lib().hdk_amg_get_cf(self.h, l, out.ctypes.data))
+        return out
+
+    def dof_func(self, l):
+        """Function labels of this rank's rows of level l (systems AMG)."""
+        out = np.empty(self.level_info(l)["rows"], dtype=np.int32)
+        check(lib().hdk_amg_get_dof_func(self.h, l, out.ctypes.data))
         return out
 
     def measure(self, l):

@@ -130,6 +130,9 @@ HYPREDRV_EXPORT_SYMBOL uint32_t HYPREDRV_LinearSystemSetStencil(HYPREDRV_t hypre
 HYPREDRV_EXPORT_SYMBOL uint32_t HYPREDRV_LinearSystemGetDevicePointers(HYPREDRV_t hypredrv, double **x_d, double **b_d);
 /* B200 extension (additive): opaque device handles for roofline instrumentation (bench.py). */
 HYPREDRV_EXPORT_SYMBOL uint32_t HYPREDRV_GetDeviceHandles(HYPREDRV_t hypredrv, void **hdk_matrix, void **hdk_amg);
+/* B200 extension (additive): the hdk_amg_params block (include/hdk.h) the next AMG setup passes to
+ * the device, after the same option checks (error bits set for unsupported combinations). */
+HYPREDRV_EXPORT_SYMBOL uint32_t HYPREDRV_PreconGetDeviceParams(HYPREDRV_t hypredrv, void *hdk_amg_params);
 
 /* ---- preconditioner / solver lifecycle --------------------------------------------------- */
 HYPREDRV_EXPORT_SYMBOL uint32_t HYPREDRV_PreconCreate(HYPREDRV_t hypredrv);                    /* :1719 */

@@ -132,6 +132,11 @@ typedef struct
    int    rand_seed;       /* 2747 */
    int    keep_transpose;  /* 1: store R = P^T explicitly */
    int    print_level;
+   /* systems AMG, unknown approach (hypre num_functions / dof_func): > 1 keeps strength and
+    * interpolation inside each function.  dof_func: host array of this rank's row labels in
+    * [0, num_functions), read during the setup only; NULL = interleaved (global row % num_functions) */
+   int            num_functions; /* 1 */
+   const int32_t *dof_func;      /* NULL */
 } hdk_amg_params;
 
 void hdk_amg_default_params(hdk_amg_params *p);
@@ -156,6 +161,8 @@ int hdk_amg_get_matrix(const hdk_amg *M, int level, int which, int32_t *rowptr_h
 int hdk_amg_get_rows(const hdk_amg *M, int level, int which, int64_t *row0, int64_t *nrows, int64_t *nnz,
                      int64_t *indptr_h, int64_t *cols_h, double *vals_h);
 int hdk_amg_get_cf(const hdk_amg *M, int level, int32_t *cf_h);
+/* function labels of this rank's rows of level l (hierarchies built with num_functions > 1) */
+int hdk_amg_get_dof_func(const hdk_amg *M, int level, int32_t *dof_h);
 int hdk_amg_get_measure(const hdk_amg *M, int level, double *measure_h);
 int hdk_amg_get_l1(const hdk_amg *M, int level, double *l1_h);
 double hdk_amg_operator_complexity(const hdk_amg *M);
