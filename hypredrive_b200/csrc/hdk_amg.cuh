@@ -11,6 +11,7 @@ struct AmgLevel
    hdk_csr_s *P = nullptr;  // n_l x n_{l+1}
    hdk_csr_s *R = nullptr;  // n_{l+1} x n_l  (P^T stored explicitly: keep_transpose)
    DevCSR     S;            // strength pattern (diag block)
+   DevCSR     S2;           // aggressive levels: second-stage strength over the first-stage C points
    int       *cf = nullptr;
    int       *f2c = nullptr; // exclusive scan of (cf > 0), n+1 entries (kept for the N > 1 slicing)
    double    *measure = nullptr;

@@ -1843,6 +1843,732 @@ int build_rap(const DevCSR &R, const DevCSR &A, const DevCSR &P, DevCSR &C, int 
 }
 
 // =====================================================================================
+// aggressive coarsening (agg_num_levels, DESIGN.md §4): second-stage strength S2 over the
+// first-stage C points (after hypre_BoomerAMGCreate2ndS), a second PMIS on S2, the combined C/F
+// marker (after hypre_BoomerAMGCorrectCFMarker2) and multipass interpolation (after
+// hypre_BoomerAMGBuildModMultipass), each pass truncated before it feeds the next.  The rule is
+// the one restated in tests/aggressive_oracle.c; the device reproduces it bit for bit.
+// =====================================================================================
+// HDK_AGG_THREAD=1: every S2 row and every pass-p product row takes the one-thread-per-row path
+// with global-scratch tables instead of the warp kernels (read once per process)
+static bool agg_force_thread()
+{
+   static int v = -1;
+   if (v < 0) { const char *e = getenv("HDK_AGG_THREAD"); v = (e && atoi(e) == 1) ? 1 : 0; }
+   return v == 1;
+}
+
+constexpr int S2_CAP = 512, S2_LIMIT = 320, S2_WARPS = 4;
+
+__global__ void k_s2_rows(const int *cf, const int *c1, int n, int *rows)
+{
+   int i = blockIdx.x * blockDim.x + threadIdx.x;
+   if (i < n && cf[i] == C_PT) rows[c1[i]] = i;
+}
+
+// One warp per first-stage C row: path counts keyed by coarse column in a shared-memory table (the
+// lanes walk the strong neighbours and their strong neighbours in any order: only the counts matter,
+// the row is sorted afterwards).  The number of keys is checked before every insert, so the table
+// holds at most S2_LIMIT + 32 keys; a row that reaches the limit is flagged for k_s2_thread_*.
+// !FILL: row lengths (entries with count >= num_paths); FILL: the ascending row.
+template <bool FILL>
+__global__ void __launch_bounds__(32 * S2_WARPS) k_s2_warp(const int *srp, const int *scol, const int *cf, const int *c1, const int *rows,
+                                                           int nc1, int num_paths, int *cnt, int *slow, const int *s2rp, int *s2col, int force_thread)
+{
+   __shared__ int s_keys[S2_WARPS * S2_CAP];
+   __shared__ int s_cnt[S2_WARPS * S2_CAP];
+   __shared__ int s_sel[S2_WARPS * (S2_LIMIT + 32)];
+   __shared__ int s_nk[S2_WARPS];
+   const int      lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+   const unsigned FULL = 0xffffffffu;
+   const int      ic = blockIdx.x * S2_WARPS + wid;
+   if (ic >= nc1) return;
+   if (!FILL && force_thread) { if (lane == 0) { slow[ic] = 1; cnt[ic] = 0; } return; }
+   if (FILL && slow[ic]) return;
+   int *keys = s_keys + wid * S2_CAP, *cnts = s_cnt + wid * S2_CAP, *sel = s_sel + wid * (S2_LIMIT + 32);
+   for (int h = lane; h < S2_CAP; h += 32) { keys[h] = -1; cnts[h] = 0; }
+   if (lane == 0) s_nk[wid] = 0;
+   __syncwarp();
+   volatile int *nk = s_nk + wid;
+   const int i = rows[ic];
+   bool overflow = false;
+   for (int k = srp[i] + lane; k < srp[i + 1] && !overflow; k += 32)
+   {
+      const int j = scol[k];
+      const int kb = (cf[j] == C_PT) ? -1 : srp[j], ke = (cf[j] == C_PT) ? 0 : srp[j + 1];
+      for (int kk = kb; kk < ke; kk++)
+      {
+         const int j2 = (kk < 0) ? j : scol[kk];
+         if (kk < 0 || (cf[j2] == C_PT && j2 != i))
+         {
+            if (*nk > S2_LIMIT) { overflow = true; break; }
+            bool isnew;
+            const int h = wt_find_or_insert(keys, S2_CAP, c1[j2], isnew);
+            atomicAdd(cnts + h, 1);
+            if (isnew) atomicAdd(s_nk + wid, 1);
+         }
+      }
+   }
+   overflow = __any_sync(FULL, overflow) || *nk > S2_LIMIT;
+   __syncwarp();
+   if (overflow) { if (!FILL && lane == 0) { slow[ic] = 1; cnt[ic] = 0; } return; }
+   int m = 0;
+   for (int h0 = 0; h0 < S2_CAP; h0 += 32)
+   {
+      const int      h = h0 + lane;
+      const bool     s = keys[h] >= 0 && cnts[h] >= num_paths;
+      const unsigned b = __ballot_sync(FULL, s);
+      if (FILL && s) sel[m + __popc(b & ((1u << lane) - 1u))] = keys[h];
+      m += __popc(b);
+   }
+   if (!FILL) { if (lane == 0) { slow[ic] = 0; cnt[ic] = m; } return; }
+   __syncwarp();
+   const int b0 = s2rp[ic];
+   for (int e = lane; e < m; e += 32)
+   {
+      const int key = sel[e];
+      int       rank = 0;
+      for (int x = 0; x < m; x++) rank += sel[x] < key;
+      s2col[b0 + rank] = key;
+   }
+}
+
+__global__ void k_s2_cap(const int *srp, const int *scol, const int *cf, const int *rows, const int *slow, int nc1, int *cap)
+{
+   int ic = blockIdx.x * blockDim.x + threadIdx.x;
+   if (ic > nc1) return;
+   int c = 0;
+   if (ic < nc1 && slow[ic])
+   {
+      const int i  = rows[ic];
+      int       ub = 0;
+      for (int k = srp[i]; k < srp[i + 1]; k++) { int j = scol[k]; ub += (cf[j] == C_PT) ? 1 : srp[j + 1] - srp[j]; }
+      c = pow2ceil(2 * ub);
+   }
+   cap[ic] = c;
+}
+
+// one thread per flagged row, (coarse column, path count) table in global scratch (int2, keys -1)
+__device__ __forceinline__ void s2_thread_table(const int *srp, const int *scol, const int *cf, const int *c1, int i, int2 *tab, int cap)
+{
+   const unsigned mask = (unsigned)cap - 1;
+   for (int k = srp[i]; k < srp[i + 1]; k++)
+   {
+      const int j  = scol[k];
+      const int kb = (cf[j] == C_PT) ? -1 : srp[j], ke = (cf[j] == C_PT) ? 0 : srp[j + 1];
+      for (int kk = kb; kk < ke; kk++)
+      {
+         const int j2 = (kk < 0) ? j : scol[kk];
+         if (kk >= 0 && (cf[j2] != C_PT || j2 == i)) continue;
+         const int key = c1[j2];
+         unsigned  h   = hslot(key, cap);
+         while (true)
+         {
+            const int t = tab[h].x;
+            if (t == key) { tab[h].y++; break; }
+            if (t == -1) { tab[h] = make_int2(key, 1); break; }
+            h = (h + 1) & mask;
+         }
+      }
+   }
+}
+__global__ void k_s2_thread_count(const int *srp, const int *scol, const int *cf, const int *c1, const int *rows, const int *slow,
+                                  int row0, int row1, const int64_t *off, int2 *tab, int num_paths, int *cnt)
+{
+   int ic = row0 + blockIdx.x * blockDim.x + threadIdx.x;
+   if (ic >= row1 || !slow[ic]) return;
+   int2 *t   = tab + (off[ic] - off[row0]);
+   int   cap = (int)(off[ic + 1] - off[ic]);
+   s2_thread_table(srp, scol, cf, c1, rows[ic], t, cap);
+   int c = 0;
+   for (int h = 0; h < cap; h++) c += (t[h].x >= 0 && t[h].y >= num_paths);
+   cnt[ic] = c;
+}
+__global__ void k_s2_thread_fill(const int *srp, const int *scol, const int *cf, const int *c1, const int *rows, const int *slow,
+                                 int row0, int row1, const int64_t *off, int2 *tab, int num_paths, const int *s2rp, int *s2col)
+{
+   int ic = row0 + blockIdx.x * blockDim.x + threadIdx.x;
+   if (ic >= row1 || !slow[ic]) return;
+   int2 *t   = tab + (off[ic] - off[row0]);
+   int   cap = (int)(off[ic + 1] - off[ic]);
+   s2_thread_table(srp, scol, cf, c1, rows[ic], t, cap);
+   int *r = s2col + s2rp[ic], m = 0;
+   for (int h = 0; h < cap; h++)
+      if (t[h].x >= 0 && t[h].y >= num_paths)
+      {
+         int key = t[h].x, x = m++;
+         while (x > 0 && r[x - 1] > key) { r[x] = r[x - 1]; x--; } // insertion sort
+         r[x] = key;
+      }
+}
+
+// first-stage C points that the second PMIS made F become -2 (hypre_BoomerAMGCorrectCFMarker2)
+__global__ void k_s2_combine(int *cf, const int *c1, const int *cf2, int n)
+{
+   int i = blockIdx.x * blockDim.x + threadIdx.x;
+   if (i < n && cf[i] == C_PT && cf2[c1[i]] == F_PT) cf[i] = -2;
+}
+
+// S2 of the first-stage C points (cf == 1, coarse index c1), rows in ascending column order
+static int build_s2(const DevCSR &S, const int *cf, const int *c1, int nc1, int num_paths, DevCSR &S2)
+{
+   int *rows, *cnt, *slow, *cap, *rp;
+   int64_t *off;
+   HDK_TRY(dalloc(&rows, (size_t)nc1 + 1));
+   HDK_TRY(dalloc(&cnt, (size_t)nc1 + 1));
+   HDK_TRY(dalloc(&slow, (size_t)nc1 + 1));
+   HDK_TRY(dalloc(&cap, (size_t)nc1 + 1));
+   HDK_TRY(dalloc(&off, (size_t)nc1 + 1));
+   HDK_TRY(dalloc(&rp, (size_t)nc1 + 1));
+   const int n = S.nrows, force = agg_force_thread() ? 1 : 0;
+   k_s2_rows<<<cdiv(n, 256), 256, 0, g.stream>>>(cf, c1, n, rows);
+   HDK_LAUNCH_CHECK();
+   k_s2_warp<false><<<cdiv(nc1, S2_WARPS), 32 * S2_WARPS, 0, g.stream>>>(S.rowptr, S.col, cf, c1, rows, nc1, num_paths, cnt, slow, nullptr, nullptr, force);
+   HDK_LAUNCH_CHECK();
+   k_s2_cap<<<cdiv(nc1 + 1, 256), 256, 0, g.stream>>>(S.rowptr, S.col, cf, rows, slow, nc1, cap);
+   HDK_LAUNCH_CHECK();
+   HDK_TRY(exclusive_scan_i64(cap, off, nc1 + 1));
+   std::vector<int> bounds;
+   int64_t          maxsz;
+   HDK_TRY(plan_chunks(off, nc1, bounds, maxsz));
+   int2 *tab;
+   HDK_TRY(dalloc(&tab, (size_t)maxsz + 4));
+   for (size_t c = 0; c + 1 < bounds.size(); c++)
+   {
+      int r0 = bounds[c], r1 = bounds[c + 1];
+      if (r1 <= r0 || maxsz == 0) continue;
+      HDK_CUDA(cudaMemsetAsync(tab, 0xFF, sizeof(int2) * ((size_t)maxsz + 4), g.stream));
+      k_s2_thread_count<<<cdiv(r1 - r0, 128), 128, 0, g.stream>>>(S.rowptr, S.col, cf, c1, rows, slow, r0, r1, off, tab, num_paths, cnt);
+      HDK_LAUNCH_CHECK();
+   }
+   HDK_CUDA(cudaMemsetAsync(cnt + nc1, 0, sizeof(int), g.stream));
+   HDK_TRY(check_fits_int32(cnt, nc1, "the second-stage strength matrix"));
+   HDK_TRY(exclusive_scan_int(cnt, rp, nc1 + 1));
+   int nnz = 0;
+   HDK_CUDA(cudaMemcpyAsync(&nnz, rp + nc1, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
+   HDK_CUDA(cudaStreamSynchronize(g.stream));
+   S2 = DevCSR();
+   S2.nrows = nc1; S2.ncols = nc1; S2.nnz = nnz; S2.rowptr = rp; S2.owns = true;
+   HDK_TRY(dalloc(&S2.col, (size_t)nnz + 8));
+   k_s2_warp<true><<<cdiv(nc1, S2_WARPS), 32 * S2_WARPS, 0, g.stream>>>(S.rowptr, S.col, cf, c1, rows, nc1, num_paths, cnt, slow, rp, S2.col, force);
+   HDK_LAUNCH_CHECK();
+   for (size_t c = 0; c + 1 < bounds.size(); c++)
+   {
+      int r0 = bounds[c], r1 = bounds[c + 1];
+      if (r1 <= r0 || maxsz == 0) continue;
+      HDK_CUDA(cudaMemsetAsync(tab, 0xFF, sizeof(int2) * ((size_t)maxsz + 4), g.stream));
+      k_s2_thread_fill<<<cdiv(r1 - r0, 128), 128, 0, g.stream>>>(S.rowptr, S.col, cf, c1, rows, slow, r0, r1, off, tab, num_paths, rp, S2.col);
+      HDK_LAUNCH_CHECK();
+   }
+   dfree(tab); dfree(rows); dfree(cnt); dfree(slow); dfree(cap); dfree(off);
+   return HDK_OK;
+}
+
+// second stage of an aggressive level: S2, PMIS on S2 (random offset 0), combined marker in cf
+static int aggressive_second_stage(AmgLevel &L, int n, const hdk_amg_params *prm, bool keep_debug)
+{
+   int *flag, *c1;
+   HDK_TRY(dalloc(&flag, (size_t)n + 1));
+   HDK_TRY(dalloc(&c1, (size_t)n + 1));
+   k_cf_flag<<<cdiv(n + 1, 256), 256, 0, g.stream>>>(L.cf, n, flag);
+   HDK_LAUNCH_CHECK();
+   HDK_TRY(exclusive_scan_int(flag, c1, n + 1));
+   int nc1 = 0;
+   HDK_CUDA(cudaMemcpyAsync(&nc1, c1 + n, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
+   HDK_CUDA(cudaStreamSynchronize(g.stream));
+   dfree(flag);
+   if (nc1 == 0) { dfree(c1); return HDK_OK; }
+   DevCSR S2;
+   HDK_TRY(build_s2(L.S, L.cf, c1, nc1, prm->agg_num_paths, S2));
+   stage_mark("s2", -1);
+   int    *cf2;
+   double *m2;
+   HDK_TRY(dalloc(&cf2, (size_t)nc1 + 1));
+   HDK_TRY(dalloc(&m2, (size_t)nc1 + 1));
+   HDK_TRY(run_pmis(S2, prm->rand_seed, 0, cf2, m2, nullptr, nullptr));
+   k_s2_combine<<<cdiv(n, 256), 256, 0, g.stream>>>(L.cf, c1, cf2, n);
+   HDK_LAUNCH_CHECK();
+   stage_mark("pmis2", -1);
+   dfree(cf2); dfree(m2); dfree(c1);
+   if (keep_debug) L.S2 = S2;
+   else csr_free(S2);
+   return HDK_OK;
+}
+
+// ---- multipass interpolation ---------------------------------------------------------------
+// pass[i]: 1 for C points, p + 1 for a point with a strong neighbour of pass p, 0 if unreached.
+// A sweep tests only == p and writes only p + 1, so it reads no value it writes.
+__global__ void k_mp_pass_init(const int *cf, int n, int *pass)
+{
+   int i = blockIdx.x * blockDim.x + threadIdx.x;
+   if (i < n) pass[i] = cf[i] > 0 ? 1 : 0;
+}
+__global__ void k_mp_pass(const int *srp, const int *scol, int n, int p, int *pass, int *assigned)
+{
+   int  i = blockIdx.x * blockDim.x + threadIdx.x;
+   bool a = false;
+   if (i < n && pass[i] == 0)
+      for (int k = srp[i]; k < srp[i + 1]; k++)
+         if (pass[scol[k]] == p) { pass[i] = p + 1; a = true; break; }
+   int c = __syncthreads_count(a);
+   if (threadIdx.x == 0 && c) atomicAdd(assigned, c);
+}
+
+// a_ij of every strong neighbour: S keeps A's column order, so both rows are walked together
+__global__ void k_mp_sval(const int *arp, const int *acol, const double *aval, const int *srp, const int *scol, int n, double *sval)
+{
+   int i = blockIdx.x * blockDim.x + threadIdx.x;
+   if (i >= n) return;
+   int ka = arp[i] + 1;
+   for (int k = srp[i]; k < srp[i + 1]; k++)
+   {
+      while (acol[ka] != scol[k]) ka++;
+      sval[k] = aval[ka++];
+   }
+}
+
+// row scalars of the pass >= 2 rows: alfa (negative couplings), beta (positive couplings); live = 0
+// for a row whose lumped diagonal is zero (empty P row)
+__global__ void k_mp_scal(const int *arp, const double *aval, const int *srp, const int *scol, const double *sval, const int *pass, int n,
+                          double *alfa, double *beta, int *live)
+{
+   int i = blockIdx.x * blockDim.x + threadIdx.x;
+   if (i >= n) return;
+   const int p = pass[i];
+   if (p < 2) { live[i] = 0; return; }
+   double nneg = 0.0, npos = 0.0, cneg = 0.0, cpos = 0.0;
+   for (int k = arp[i] + 1; k < arp[i + 1]; k++)
+   {
+      double v = aval[k];
+      if (v < 0) nneg = __dadd_rn(nneg, v);
+      else npos = __dadd_rn(npos, v);
+   }
+   for (int k = srp[i]; k < srp[i + 1]; k++)
+      if (pass[scol[k]] == p - 1)
+      {
+         double v = sval[k];
+         if (v < 0) cneg = __dadd_rn(cneg, v);
+         else cpos = __dadd_rn(cpos, v);
+      }
+   double d = aval[arp[i]];
+   if (cpos == 0.0) d = __dadd_rn(d, npos);
+   live[i] = d != 0.0;
+   alfa[i] = cneg != 0.0 ? __ddiv_rn(__ddiv_rn(nneg, cneg), d) : 0.0;
+   beta[i] = cpos != 0.0 ? __ddiv_rn(__ddiv_rn(npos, cpos), d) : 0.0;
+}
+__device__ __forceinline__ double mp_weight(double a, double al, double be) { return a < 0 ? -__dmul_rn(al, a) : -__dmul_rn(be, a); }
+
+// rows of pass p in row order (list) and every row's position in the block of its own pass (slot)
+__global__ void k_mp_flag(const int *pass, int n, int p, int *flag)
+{
+   int i = blockIdx.x * blockDim.x + threadIdx.x;
+   if (i <= n) flag[i] = (i < n && pass[i] == p) ? 1 : 0;
+}
+__global__ void k_mp_list(const int *pass, const int *pos, int n, int p, int *list, int *slot)
+{
+   int i = blockIdx.x * blockDim.x + threadIdx.x;
+   if (i < n && pass[i] == p) { list[pos[i]] = i; slot[i] = pos[i]; }
+}
+
+// pass 2: one thread per row, columns of the strong C neighbours in S order
+template <bool FILL>
+__global__ void k_mp_pass2(const int *list, int m, const int *srp, const int *scol, const double *sval, const int *pass, const double *alfa,
+                           const double *beta, const int *live, const int *f2c, int *len, const int *qrp, int *qcol, double *qval)
+{
+   int r = blockIdx.x * blockDim.x + threadIdx.x;
+   if (r > m) return;
+   if (r == m) { if (!FILL) len[m] = 0; return; }
+   const int i = list[r];
+   if (!live[i]) { if (!FILL) len[r] = 0; return; }
+   const double al = alfa[i], be = beta[i];
+   int c = FILL ? qrp[r] : 0;
+   for (int k = srp[i]; k < srp[i + 1]; k++)
+   {
+      const int j = scol[k];
+      if (pass[j] != 1) continue;
+      if (FILL) { qcol[c] = f2c[j]; qval[c] = mp_weight(sval[k], al, be); }
+      c++;
+   }
+   if (!FILL) len[r] = c;
+}
+
+// pass p >= 3: P_i = sum over the strong pass-(p-1) neighbours j of w_ij * P_j (truncated rows of the
+// previous block).  One warp per row walks the product stream 32 products at a time in the order
+// j in S_i, then P_j in stored order; lanes that hit the same column are grouped with match.any, the
+// group leader takes the slot (new columns in lane order = discovery order) and adds the group's
+// products in lane order, as in k_rap_warp.  Rows with more than MP_LIMIT columns are flagged (slow)
+// for the one-thread-per-row kernels.
+constexpr int MP_CAP = 512, MP_LIMIT = 320, MP_WARPS = 4;
+
+template <bool FILL>
+__global__ void __launch_bounds__(32 * MP_WARPS) k_mp_warp(const int *list, int m, const int *srp, const int *scol, const double *sval,
+                                                           const int *pass, int p, const double *alfa, const double *beta, const int *live,
+                                                           const int *slot, const int *qrp, const int *qcol, const double *qval,
+                                                           int *cnt, int *slow, const int *prp, int *pcol, double *pval, int force_thread)
+{
+   __shared__ int    s_keys[MP_WARPS * MP_CAP];
+   __shared__ int    s_idx[MP_WARPS * MP_CAP];
+   __shared__ double s_vals[MP_WARPS * MP_CAP];
+   const int      lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+   const unsigned FULL = 0xffffffffu;
+   const int      r = blockIdx.x * MP_WARPS + wid;
+   if (r >= m) return;
+   if (!FILL && force_thread) { if (lane == 0) { slow[r] = 1; cnt[r] = 0; } return; }
+   if (FILL && slow[r]) return;
+   const int i = list[r];
+   if (!live[i]) { if (!FILL && lane == 0) { slow[r] = 0; cnt[r] = 0; } return; }
+   int    *keys = s_keys + wid * MP_CAP, *idx = s_idx + wid * MP_CAP;
+   double *vals = s_vals + wid * MP_CAP;
+   for (int h = lane; h < MP_CAP; h += 32) keys[h] = -1;
+   __syncwarp();
+   const double al = alfa[i], be = beta[i];
+   const int    send = srp[i + 1];
+   int          count = 0;
+   bool         overflow = false;
+   for (int sb = srp[i]; sb < send && !overflow; sb += 32)
+   {
+      const int  k  = sb + lane;
+      const int  j  = k < send ? scol[k] : 0;
+      const bool in = k < send && pass[j] == p - 1;
+      double     w  = 0.0;
+      int        ps = 0, pl = 0;
+      if (in)
+      {
+         if (FILL) w = mp_weight(sval[k], al, be);
+         const int s = slot[j];
+         ps = qrp[s]; pl = qrp[s + 1] - ps;
+      }
+      int incl = pl;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) { int u = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += u; }
+      const int excl = incl - pl, Tc = __shfl_sync(FULL, incl, 31);
+      for (int q0 = 0; q0 < Tc; q0 += 32)
+      {
+         const int  q = q0 + lane;
+         const bool act = q < Tc;
+         int lo = 0, hi = 31; // smallest lane m with incl[m] > q
+#pragma unroll
+         for (int s = 0; s < 5; s++)
+         {
+            int mid = (lo + hi) >> 1;
+            int v   = __shfl_sync(FULL, incl, mid);
+            if (v > q) hi = mid; else lo = mid + 1;
+         }
+         const int    src = lo;
+         const int    j3  = q - __shfl_sync(FULL, excl, src);
+         const int    psm = __shfl_sync(FULL, ps, src);
+         const double wm  = __shfl_sync(FULL, w, src);
+         const int    key = act ? qcol[psm + j3] : (-2 - lane);
+         const double prod = (FILL && act) ? __dmul_rn(wm, qval[psm + j3]) : 0.0;
+         const unsigned grp = __match_any_sync(FULL, key);
+         const bool leader = act && (lane == __ffs(grp) - 1);
+         bool isnew = false;
+         int  h = 0;
+         if (leader) h = wt_find_or_insert(keys, MP_CAP, key, isnew);
+         const unsigned newmask = __ballot_sync(FULL, leader && isnew);
+         if (FILL && leader && isnew) idx[h] = count + __popc(newmask & ((1u << lane) - 1u));
+         count += __popc(newmask);
+         if (count > MP_LIMIT) overflow = true;
+         if (FILL)
+         {
+            const int maxc = (int)__reduce_max_sync(FULL, leader ? (unsigned)__popc(grp) : 0u);
+            double    acc = 0.0;
+            bool      first = true;
+            unsigned  rem = leader ? grp : 0u;
+            for (int s = 0; s < maxc; s++)
+            {
+               int    from = rem ? (__ffs(rem) - 1) : lane;
+               double v    = __shfl_sync(FULL, prod, from);
+               if (rem)
+               {
+                  if (first) { acc = isnew ? v : __dadd_rn(vals[h], v); first = false; }
+                  else acc = __dadd_rn(acc, v);
+                  rem &= rem - 1u;
+               }
+            }
+            if (leader) vals[h] = acc;
+         }
+         __syncwarp();
+         if (overflow) break;
+      }
+   }
+   if (!FILL) { if (lane == 0) { slow[r] = overflow ? 1 : 0; cnt[r] = overflow ? 0 : count; } return; }
+   const int b = prp[r];
+   for (int h = lane; h < MP_CAP; h += 32)
+      if (keys[h] >= 0) { pcol[b + idx[h]] = keys[h]; pval[b + idx[h]] = vals[h]; }
+}
+
+__global__ void k_mp_cap(const int *list, int m, const int *srp, const int *scol, const int *pass, int p, const int *live,
+                         const int *slot, const int *qrp, const int *slow, int *cap)
+{
+   int r = blockIdx.x * blockDim.x + threadIdx.x;
+   if (r > m) return;
+   int c = 0;
+   if (r < m && slow[r] && live[list[r]])
+   {
+      const int i  = list[r];
+      int       ub = 0;
+      for (int k = srp[i]; k < srp[i + 1]; k++)
+      {
+         const int j = scol[k];
+         if (pass[j] == p - 1) ub += qrp[slot[j] + 1] - qrp[slot[j]];
+      }
+      c = pow2ceil(2 * ub);
+   }
+   cap[r] = c;
+}
+__global__ void k_mp_thread_count(const int *list, const int *srp, const int *scol, const int *pass, int p, const int *slot,
+                                  const int *qrp, const int *qcol, const int *slow, int row0, int row1, const int64_t *off, int *keys, int *cnt)
+{
+   int r = row0 + blockIdx.x * blockDim.x + threadIdx.x;
+   if (r >= row1 || !slow[r]) return;
+   int *tab = keys + (off[r] - off[row0]);
+   int  cap = (int)(off[r + 1] - off[r]), c = 0;
+   if (cap > 0)
+   {
+      const int i = list[r];
+      for (int k = srp[i]; k < srp[i + 1]; k++)
+      {
+         const int j = scol[k];
+         if (pass[j] != p - 1) continue;
+         const int s = slot[j];
+         for (int t = qrp[s]; t < qrp[s + 1]; t++) if (hset_insert(tab, cap, qcol[t])) c++;
+      }
+   }
+   cnt[r] = c;
+}
+__global__ void k_mp_thread_fill(const int *list, const int *srp, const int *scol, const double *sval, const int *pass, int p,
+                                 const double *alfa, const double *beta, const int *slot, const int *qrp, const int *qcol, const double *qval,
+                                 const int *slow, int row0, int row1, const int64_t *off, int2 *htab, const int *prp, int *pcol, double *pval)
+{
+   int r = row0 + blockIdx.x * blockDim.x + threadIdx.x;
+   if (r >= row1 || !slow[r]) return;
+   int2 *tab = htab + (off[r] - off[row0]);
+   int   cap = (int)(off[r + 1] - off[r]);
+   if (cap == 0) return;
+   const int    i = list[r];
+   const double al = alfa[i], be = beta[i];
+   int          c = prp[r];
+   for (int k = srp[i]; k < srp[i + 1]; k++)
+   {
+      const int j = scol[k];
+      if (pass[j] != p - 1) continue;
+      const double w = mp_weight(sval[k], al, be);
+      const int    s = slot[j];
+      for (int t = qrp[s]; t < qrp[s + 1]; t++)
+      {
+         const double prod = __dmul_rn(w, qval[t]);
+         const int    x    = hmap_insert(tab, cap, qcol[t], c);
+         if (x == -1) { pcol[c] = qcol[t]; pval[c] = prod; c++; }
+         else pval[x] = __dadd_rn(pval[x], prod);
+      }
+   }
+}
+
+// final P: C rows (one entry 1.0 at f2c[i]) and every pass block's rows scattered to their fine row
+__global__ void k_mp_len_c(const int *pass, int n, int *len)
+{
+   int i = blockIdx.x * blockDim.x + threadIdx.x;
+   if (i <= n) len[i] = (i < n && pass[i] == 1) ? 1 : 0;
+}
+__global__ void k_mp_len_block(const int *list, int m, const int *qrp, int *len)
+{
+   int r = blockIdx.x * blockDim.x + threadIdx.x;
+   if (r < m) len[list[r]] = qrp[r + 1] - qrp[r];
+}
+__global__ void k_mp_copy_c(const int *pass, const int *f2c, const int *prp, int n, int *pcol, double *pval)
+{
+   int i = blockIdx.x * blockDim.x + threadIdx.x;
+   if (i < n && pass[i] == 1) { pcol[prp[i]] = f2c[i]; pval[prp[i]] = 1.0; }
+}
+__global__ void k_mp_copy_block(const int *list, int m, const int *qrp, const int *qcol, const double *qval, const int *prp, int *pcol, double *pval)
+{
+   int r = blockIdx.x * blockDim.x + threadIdx.x;
+   if (r >= m) return;
+   const int b = prp[list[r]];
+   for (int t = qrp[r]; t < qrp[r + 1]; t++) { pcol[b + t - qrp[r]] = qcol[t]; pval[b + t - qrp[r]] = qval[t]; }
+}
+
+// rows of pass p >= 3 into the block Q (rows in list order), from the previous block Qp
+static int mp_products(const int *list, int m, const DevCSR &S, const double *sval, const int *pass, int p, const double *alfa,
+                       const double *beta, const int *live, const int *slot, const DevCSR &Qp, DevCSR &Q)
+{
+   int *cnt, *slow, *cap, *rp;
+   int64_t *off;
+   HDK_TRY(dalloc(&cnt, (size_t)m + 1));
+   HDK_TRY(dalloc(&slow, (size_t)m + 1));
+   HDK_TRY(dalloc(&cap, (size_t)m + 1));
+   HDK_TRY(dalloc(&off, (size_t)m + 1));
+   HDK_TRY(dalloc(&rp, (size_t)m + 1));
+   const int force = agg_force_thread() ? 1 : 0;
+   k_mp_warp<false><<<cdiv(m, MP_WARPS), 32 * MP_WARPS, 0, g.stream>>>(list, m, S.rowptr, S.col, sval, pass, p, alfa, beta, live, slot,
+                                                                       Qp.rowptr, Qp.col, Qp.val, cnt, slow, nullptr, nullptr, nullptr, force);
+   HDK_LAUNCH_CHECK();
+   k_mp_cap<<<cdiv(m + 1, 256), 256, 0, g.stream>>>(list, m, S.rowptr, S.col, pass, p, live, slot, Qp.rowptr, slow, cap);
+   HDK_LAUNCH_CHECK();
+   HDK_TRY(exclusive_scan_i64(cap, off, m + 1));
+   std::vector<int> bounds;
+   int64_t          maxsz;
+   HDK_TRY(plan_chunks(off, m, bounds, maxsz));
+   {
+      int *keys;
+      HDK_TRY(dalloc(&keys, (size_t)maxsz + 4));
+      for (size_t c = 0; c + 1 < bounds.size(); c++)
+      {
+         int r0 = bounds[c], r1 = bounds[c + 1];
+         if (r1 <= r0 || maxsz == 0) continue;
+         HDK_CUDA(cudaMemsetAsync(keys, 0xFF, sizeof(int) * ((size_t)maxsz + 4), g.stream));
+         k_mp_thread_count<<<cdiv(r1 - r0, 128), 128, 0, g.stream>>>(list, S.rowptr, S.col, pass, p, slot, Qp.rowptr, Qp.col, slow, r0, r1, off, keys, cnt);
+         HDK_LAUNCH_CHECK();
+      }
+      dfree(keys);
+   }
+   HDK_CUDA(cudaMemsetAsync(cnt + m, 0, sizeof(int), g.stream));
+   HDK_TRY(check_fits_int32(cnt, m, "the interpolation operator"));
+   HDK_TRY(exclusive_scan_int(cnt, rp, m + 1));
+   int nnz = 0;
+   HDK_CUDA(cudaMemcpyAsync(&nnz, rp + m, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
+   HDK_CUDA(cudaStreamSynchronize(g.stream));
+   Q = DevCSR();
+   Q.nrows = m; Q.ncols = Qp.ncols; Q.nnz = nnz; Q.rowptr = rp; Q.owns = true;
+   HDK_TRY(dalloc(&Q.col, (size_t)nnz + 8));
+   HDK_TRY(dalloc(&Q.val, (size_t)nnz + 8));
+   k_mp_warp<true><<<cdiv(m, MP_WARPS), 32 * MP_WARPS, 0, g.stream>>>(list, m, S.rowptr, S.col, sval, pass, p, alfa, beta, live, slot,
+                                                                      Qp.rowptr, Qp.col, Qp.val, cnt, slow, rp, Q.col, Q.val, force);
+   HDK_LAUNCH_CHECK();
+   {
+      int2 *htab;
+      HDK_TRY(dalloc(&htab, (size_t)maxsz + 4));
+      for (size_t c = 0; c + 1 < bounds.size(); c++)
+      {
+         int r0 = bounds[c], r1 = bounds[c + 1];
+         if (r1 <= r0 || maxsz == 0) continue;
+         HDK_CUDA(cudaMemsetAsync(htab, 0xFF, sizeof(int2) * ((size_t)maxsz + 4), g.stream));
+         k_mp_thread_fill<<<cdiv(r1 - r0, 128), 128, 0, g.stream>>>(list, S.rowptr, S.col, sval, pass, p, alfa, beta, slot, Qp.rowptr, Qp.col,
+                                                                    Qp.val, slow, r0, r1, off, htab, rp, Q.col, Q.val);
+         HDK_LAUNCH_CHECK();
+      }
+      dfree(htab);
+   }
+   dfree(cnt); dfree(slow); dfree(cap); dfree(off);
+   return HDK_OK;
+}
+
+// multipass interpolation of an aggressive level (cf: combined marker, f2c: scan of cf > 0)
+static int build_multipass(const DevCSR &A, const DevCSR &S, int *cf, const int *f2c, int nc, int max_elmts, double trunc_factor, DevCSR &P)
+{
+   const int n = A.nrows;
+   int *pass, *slot, *live, *flag, *pos, *len;
+   double *sval, *alfa, *beta;
+   HDK_TRY(dalloc(&pass, (size_t)n + 1));
+   HDK_TRY(dalloc(&slot, (size_t)n + 1));
+   HDK_TRY(dalloc(&live, (size_t)n + 1));
+   HDK_TRY(dalloc(&flag, (size_t)n + 1));
+   HDK_TRY(dalloc(&pos, (size_t)n + 1));
+   HDK_TRY(dalloc(&len, (size_t)n + 1));
+   HDK_TRY(dalloc(&sval, (size_t)S.nnz + 1));
+   HDK_TRY(dalloc(&alfa, (size_t)n + 1));
+   HDK_TRY(dalloc(&beta, (size_t)n + 1));
+   int *assigned = reinterpret_cast<int *>(g.dscal + S_TMP3);
+   k_mp_pass_init<<<cdiv(n, 256), 256, 0, g.stream>>>(cf, n, pass);
+   HDK_LAUNCH_CHECK();
+   int maxp = 1;
+   for (int p = 1;; p++)
+   {
+      int h = 0;
+      HDK_CUDA(cudaMemsetAsync(assigned, 0, sizeof(int), g.stream));
+      k_mp_pass<<<cdiv(n, 256), 256, 0, g.stream>>>(S.rowptr, S.col, n, p, pass, assigned);
+      HDK_LAUNCH_CHECK();
+      HDK_CUDA(cudaMemcpyAsync(&h, assigned, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
+      HDK_CUDA(cudaStreamSynchronize(g.stream));
+      if (h == 0) break;
+      maxp = p + 1;
+   }
+   k_mp_sval<<<cdiv(n, 256), 256, 0, g.stream>>>(A.rowptr, A.col, A.val, S.rowptr, S.col, n, sval);
+   HDK_LAUNCH_CHECK();
+   k_mp_scal<<<cdiv(n, 256), 256, 0, g.stream>>>(A.rowptr, A.val, S.rowptr, S.col, sval, pass, n, alfa, beta, live);
+   HDK_LAUNCH_CHECK();
+   // one block of rows per pass >= 2, truncated before it feeds the next pass
+   std::vector<DevCSR> Q((size_t)maxp + 1);
+   std::vector<int *>  lists((size_t)maxp + 1, nullptr);
+   std::vector<int>    ms((size_t)maxp + 1, 0);
+   int rc = HDK_OK;
+   for (int p = 2; p <= maxp && rc == HDK_OK; p++)
+   {
+      k_mp_flag<<<cdiv(n + 1, 256), 256, 0, g.stream>>>(pass, n, p, flag);
+      HDK_LAUNCH_CHECK();
+      HDK_TRY(exclusive_scan_int(flag, pos, n + 1));
+      int m = 0;
+      HDK_CUDA(cudaMemcpyAsync(&m, pos + n, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
+      HDK_CUDA(cudaStreamSynchronize(g.stream));
+      ms[(size_t)p] = m;
+      HDK_TRY(dalloc(&lists[(size_t)p], (size_t)m + 1));
+      k_mp_list<<<cdiv(n, 256), 256, 0, g.stream>>>(pass, pos, n, p, lists[(size_t)p], slot);
+      HDK_LAUNCH_CHECK();
+      DevCSR &B = Q[(size_t)p];
+      if (p == 2)
+      {
+         int *rp;
+         HDK_TRY(dalloc(&rp, (size_t)m + 1));
+         k_mp_pass2<false><<<cdiv(m + 1, 256), 256, 0, g.stream>>>(lists[2], m, S.rowptr, S.col, sval, pass, alfa, beta, live, f2c, len,
+                                                                   nullptr, nullptr, nullptr);
+         HDK_LAUNCH_CHECK();
+         HDK_TRY(exclusive_scan_int(len, rp, m + 1));
+         int nnz = 0;
+         HDK_CUDA(cudaMemcpyAsync(&nnz, rp + m, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
+         HDK_CUDA(cudaStreamSynchronize(g.stream));
+         B.nrows = m; B.ncols = nc; B.nnz = nnz; B.rowptr = rp; B.owns = true;
+         HDK_TRY(dalloc(&B.col, (size_t)nnz + 8));
+         HDK_TRY(dalloc(&B.val, (size_t)nnz + 8));
+         k_mp_pass2<true><<<cdiv(m + 1, 256), 256, 0, g.stream>>>(lists[2], m, S.rowptr, S.col, sval, pass, alfa, beta, live, f2c, nullptr,
+                                                                  rp, B.col, B.val);
+         HDK_LAUNCH_CHECK();
+      }
+      else HDK_TRY(mp_products(lists[(size_t)p], m, S, sval, pass, p, alfa, beta, live, slot, Q[(size_t)p - 1], B));
+      if (trunc_factor > 0.0 || max_elmts > 0) HDK_TRY(interp_truncate(B, trunc_factor, max_elmts));
+   }
+   // scatter: C rows, then every block to its fine rows
+   k_mp_len_c<<<cdiv(n + 1, 256), 256, 0, g.stream>>>(pass, n, len);
+   HDK_LAUNCH_CHECK();
+   for (int p = 2; p <= maxp; p++)
+      if (ms[(size_t)p] > 0)
+      {
+         k_mp_len_block<<<cdiv(ms[(size_t)p], 256), 256, 0, g.stream>>>(lists[(size_t)p], ms[(size_t)p], Q[(size_t)p].rowptr, len);
+         HDK_LAUNCH_CHECK();
+      }
+   HDK_TRY(check_fits_int32(len, n, "the interpolation operator"));
+   int *prp;
+   HDK_TRY(dalloc(&prp, (size_t)n + 1));
+   HDK_TRY(exclusive_scan_int(len, prp, n + 1));
+   int nnzP = 0;
+   HDK_CUDA(cudaMemcpyAsync(&nnzP, prp + n, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
+   HDK_CUDA(cudaStreamSynchronize(g.stream));
+   P = DevCSR();
+   P.nrows = n; P.ncols = nc; P.nnz = nnzP; P.rowptr = prp; P.owns = true;
+   HDK_TRY(dalloc(&P.col, (size_t)nnzP + 8));
+   HDK_TRY(dalloc(&P.val, (size_t)nnzP + 8));
+   HDK_CUDA(cudaMemsetAsync(P.col + nnzP, 0, sizeof(int) * 8, g.stream));
+   HDK_CUDA(cudaMemsetAsync(P.val + nnzP, 0, sizeof(double) * 8, g.stream));
+   k_mp_copy_c<<<cdiv(n, 256), 256, 0, g.stream>>>(pass, f2c, prp, n, P.col, P.val);
+   HDK_LAUNCH_CHECK();
+   for (int p = 2; p <= maxp; p++)
+   {
+      if (ms[(size_t)p] > 0)
+      {
+         const DevCSR &B = Q[(size_t)p];
+         k_mp_copy_block<<<cdiv(ms[(size_t)p], 256), 256, 0, g.stream>>>(lists[(size_t)p], ms[(size_t)p], B.rowptr, B.col, B.val, prp, P.col, P.val);
+         HDK_LAUNCH_CHECK();
+      }
+      csr_free(Q[(size_t)p]);
+      dfree(lists[(size_t)p]);
+   }
+   k_cf_reset_sf<<<cdiv(n, 256), 256, 0, g.stream>>>(cf, n);
+   HDK_LAUNCH_CHECK();
+   dfree(pass); dfree(slot); dfree(live); dfree(flag); dfree(pos); dfree(len); dfree(sval); dfree(alfa); dfree(beta);
+   return rc;
+}
+
+// =====================================================================================
 // l1 norms (hypre_ParCSRComputeL1Norms): option 1 full row l1 norm (relax 18);
 // option 4 truncated l1 = |a_ii| + 0.5*sum_offd|a_ij| (relax 8/13/14); option 5 diagonal
 // =====================================================================================
@@ -2115,6 +2841,7 @@ void hdk_amg_default_params(hdk_amg_params *p)
    p->relax_weight = p->outer_weight = 1.0;
    p->rand_seed = 2747; p->keep_transpose = 1; p->print_level = 0;
    p->num_functions = 1; p->dof_func = NULL;
+   p->agg_num_levels = 0; p->agg_num_paths = 1; p->agg_interp_type = 4; p->agg_max_nnz_row = 0; p->agg_trunc_factor = 0.0;
 }
 
 int hdk_amg_destroy(hdk_amg *M)
@@ -2126,7 +2853,7 @@ int hdk_amg_destroy(hdk_amg *M)
       {
          if (L.owns_A) destroy_local(L.A);
          destroy_local(L.P); destroy_local(L.R);
-         csr_free(L.S); csr_free(L.L);
+         csr_free(L.S); csr_free(L.S2); csr_free(L.L);
          dfree(L.cf); dfree(L.measure); dfree(L.f2c); dfree(L.dof);
          if (L.l1_up != L.l1_down) dfree(L.l1_up);
          dfree(L.l1_down);
@@ -2247,6 +2974,8 @@ int setup_serial(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk_amg_s **out
       stage_mark("pmis", level);
       dfree(meas);
       if (rc) break;
+      const bool agg = level < prm->agg_num_levels;
+      if (agg && (rc = aggressive_second_stage(L, n, prm, M->keep_debug))) break;
       int *flag, *f2c;
       if ((rc = dalloc(&flag, (size_t)n + 1))) break;
       if ((rc = dalloc(&f2c, (size_t)n + 1))) break;
@@ -2259,7 +2988,8 @@ int setup_serial(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk_amg_s **out
       dfree(flag);
       if (nc == 0 || nc == n || nc < prm->min_coarse_size) { dfree(f2c); break; }
       DevCSR P, R, C;
-      rc = build_interp(A.diag, L.S, L.cf, f2c, nc, prm->max_nnz_row, prm->trunc_factor, P, -1, -1, sys ? L.dof : nullptr);
+      if (agg) rc = build_multipass(A.diag, L.S, L.cf, f2c, nc, prm->agg_max_nnz_row, prm->agg_trunc_factor, P);
+      else rc = build_interp(A.diag, L.S, L.cf, f2c, nc, prm->max_nnz_row, prm->trunc_factor, P, -1, -1, sys ? L.dof : nullptr);
       stage_mark("interp", level);
       if (rc == HDK_OK && sys && (rc = dalloc(&dof_c, (size_t)nc + 1)) == HDK_OK)
       {
@@ -2534,7 +3264,7 @@ static int setup_distributed(const hdk_csr_s *A0, const hdk_amg_params *prm, hdk
          if (Lg.owns_A) { destroy_local(Lg.A); Lg.A = nullptr; Lg.owns_A = false; }
          destroy_local(Lg.P); Lg.P = nullptr;
          destroy_local(Lg.R); Lg.R = nullptr;
-         csr_free(Lg.S); csr_free(Lg.L);
+         csr_free(Lg.S); csr_free(Lg.S2); csr_free(Lg.L);
          dfree(Lg.cf); Lg.cf = nullptr; dfree(Lg.measure); Lg.measure = nullptr; dfree(Lg.f2c); Lg.f2c = nullptr;
          dfree(Lg.dof); Lg.dof = nullptr;
          if (Lg.l1_up != Lg.l1_down) dfree(Lg.l1_up);
@@ -2556,15 +3286,28 @@ int hdk_amg_setup(const hdk_csr *A0, const hdk_amg_params *prm, hdk_amg **out)
    if (prm->interp_type != 6) return set_error(HDK_ERR_UNSUPPORTED, "interpolation type %d: only extended+i (6) has a device kernel", prm->interp_type);
    if (prm->trunc_factor < 0.0 || prm->trunc_factor >= 1.0) return set_error(HDK_ERR_INVALID, "interpolation trunc_factor must be in [0, 1)");
    if (prm->num_functions < 1) return set_error(HDK_ERR_INVALID, "num_functions must be at least 1 (got %d)", prm->num_functions);
+   if (prm->agg_num_levels < 0) return set_error(HDK_ERR_INVALID, "agg_num_levels must be at least 0 (got %d)", prm->agg_num_levels);
+   const bool agg = prm->agg_num_levels > 0;
+   if (agg)
+   {
+      if (prm->agg_num_paths < 1) return set_error(HDK_ERR_INVALID, "agg_num_paths must be at least 1 (got %d)", prm->agg_num_paths);
+      if (prm->agg_max_nnz_row < 0) return set_error(HDK_ERR_INVALID, "agg_max_nnz_row must be at least 0 (got %d)", prm->agg_max_nnz_row);
+      if (!(prm->agg_trunc_factor >= 0.0 && prm->agg_trunc_factor < 1.0)) return set_error(HDK_ERR_INVALID, "agg_trunc_factor must be in [0, 1)");
+      if (prm->agg_interp_type != 4)
+         return set_error(HDK_ERR_UNSUPPORTED, "aggressive interpolation type %d: only multipass (4) has a device kernel", prm->agg_interp_type);
+      if (prm->num_functions > 1)
+         return set_error(HDK_ERR_UNSUPPORTED, "aggressive coarsening with num_functions = %d has no device setup", prm->num_functions);
+   }
    g_timing = getenv("HDK_SETUP_TIMING") && atoi(getenv("HDK_SETUP_TIMING")) == 1;
    // row-distributed setup (hdk_amg_dist.cu); HDK_SETUP_REPLICATED=1 selects the round-1 scheme that
    // rebuilds the global hierarchy on every rank (kept for comparison)
    const bool replicated = getenv("HDK_SETUP_REPLICATED") && atoi(getenv("HDK_SETUP_REPLICATED")) == 1;
    const bool force_dist = getenv("HDK_SETUP_DIST_FORCE") && atoi(getenv("HDK_SETUP_DIST_FORCE")) == 1;
-   // systems AMG has no row-distributed setup yet: N > 1 rebuilds the global hierarchy on every rank
+   // systems AMG and aggressive coarsening have no row-distributed setup yet: N > 1 rebuilds the
+   // global hierarchy on every rank
    const bool sys = prm->num_functions > 1;
-   if (g.nranks > 1 && (replicated || sys)) return setup_distributed(A0, prm, out);
-   if (!sys && (g.nranks > 1 || (force_dist && A0->orig_indptr))) return setup_distributed_rows(A0, prm, out);
+   if (g.nranks > 1 && (replicated || sys || agg)) return setup_distributed(A0, prm, out);
+   if (!sys && !agg && (g.nranks > 1 || (force_dist && A0->orig_indptr))) return setup_distributed_rows(A0, prm, out);
    return setup_serial(A0, prm, out, false, -1);
 }
 
@@ -2603,6 +3346,7 @@ int hdk_amg_get_matrix(const hdk_amg *M, int level, int which, int32_t *rowptr_h
    else if (which == 1 && L.P) D = &L.P->diag;
    else if (which == 2 && L.R) D = &L.R->diag;
    else if (which == 3 && L.S.rowptr) D = &L.S;
+   else if (which == 4 && L.S2.rowptr) D = &L.S2;
    if (!D) return set_error(HDK_ERR_INVALID, "matrix %d not available on level %d", which, level);
    if (rowptr_h) HDK_CUDA(cudaMemcpyAsync(rowptr_h, D->rowptr, sizeof(int) * ((size_t)D->nrows + 1), cudaMemcpyDeviceToHost, g.stream));
    if (col_h && D->nnz) HDK_CUDA(cudaMemcpyAsync(col_h, D->col, sizeof(int) * (size_t)D->nnz, cudaMemcpyDeviceToHost, g.stream));

@@ -612,10 +612,14 @@ void hd_amg_to_hdk(const hd_amg_args *a, hdk_amg_params *p)
    p->relax_weight = a->weight; p->outer_weight = a->outer_weight;
    p->keep_transpose = a->keep_transpose; p->print_level = a->print_level;
    p->num_functions = a->num_functions;
+   p->agg_num_levels = a->agg_num_levels; p->agg_num_paths = a->agg_num_paths;
+   p->agg_interp_type = a->agg_prolongation_type; p->agg_max_nnz_row = a->agg_max_nnz_row;
+   p->agg_trunc_factor = a->agg_trunc_factor;
 }
 
 /* systems AMG (num_functions > 1) runs hypre's unknown approach only: the nodal approach and
- * filter_functions would otherwise be ignored silently, so they are rejected */
+ * filter_functions would otherwise be ignored silently, so they are rejected; so are the aggressive
+ * coarsening options the device setup cannot honour */
 int hd_amg_check(const hd_amg_args *a)
 {
    int bad = 0;
@@ -636,6 +640,46 @@ int hd_amg_check(const hd_amg_args *a)
       hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
       hd_err_msg("amg:coarsening:filter_functions is not supported with num_functions = %d", a->num_functions);
       bad = 1;
+   }
+   /* aggressive coarsening: the keys only matter with num_levels > 0 */
+   if (a->agg_num_levels < 0)
+   {
+      hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+      hd_err_msg("amg:aggressive:num_levels must be at least 0 (got %d)", a->agg_num_levels);
+      bad = 1;
+   }
+   if (a->agg_num_levels > 0)
+   {
+      if (a->agg_num_paths < 1)
+      {
+         hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+         hd_err_msg("amg:aggressive:num_paths must be at least 1 (got %d)", a->agg_num_paths);
+         bad = 1;
+      }
+      if (a->agg_max_nnz_row < 0)
+      {
+         hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+         hd_err_msg("amg:aggressive:max_nnz_row must be at least 0 (got %d)", a->agg_max_nnz_row);
+         bad = 1;
+      }
+      if (!(a->agg_trunc_factor >= 0.0 && a->agg_trunc_factor < 1.0))
+      {
+         hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+         hd_err_msg("amg:aggressive:trunc_factor must be in [0, 1) (got %g)", a->agg_trunc_factor);
+         bad = 1;
+      }
+      if (a->agg_prolongation_type != 4)
+      {
+         hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+         hd_err_msg("amg:aggressive:prolongation_type %d is not supported: only multipass (4) has a device setup", a->agg_prolongation_type);
+         bad = 1;
+      }
+      if (a->num_functions > 1)
+      {
+         hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+         hd_err_msg("amg:aggressive:num_levels = %d is not supported with num_functions = %d", a->agg_num_levels, a->num_functions);
+         bad = 1;
+      }
    }
    return bad;
 }

@@ -27,7 +27,9 @@ class AmgParams(C.Structure):
                 ("sweeps_down", C.c_int), ("sweeps_up", C.c_int), ("sweeps_coarse", C.c_int),
                 ("relax_weight", C.c_double), ("outer_weight", C.c_double), ("rand_seed", C.c_int),
                 ("keep_transpose", C.c_int), ("print_level", C.c_int),
-                ("num_functions", C.c_int), ("dof_func", C.POINTER(C.c_int32))]
+                ("num_functions", C.c_int), ("dof_func", C.POINTER(C.c_int32)),
+                ("agg_num_levels", C.c_int), ("agg_num_paths", C.c_int), ("agg_interp_type", C.c_int),
+                ("agg_max_nnz_row", C.c_int), ("agg_trunc_factor", C.c_double)]
 
 
 class Krylov(C.Structure):
@@ -259,8 +261,17 @@ class DAmg:
         return [(self.level_info(l)["rows"], self.level_info(l)["nnz_A"]) for l in range(self.nlev)]
 
     def matrix(self, l, which):
-        """which: 'A', 'P', 'R', 'S' -> (rowptr, col, val) in storage order."""
-        code = {"A": 0, "P": 1, "R": 2, "S": 3}[which]
+        """which: 'A', 'P', 'R', 'S', 'S2' -> (rowptr, col, val) in storage order.  'S2' is the
+        second-stage strength of an aggressive level over its first-stage C points (amg_keep_debug)."""
+        code = {"A": 0, "P": 1, "R": 2, "S": 3, "S2": 4}[which]
+        if which == "S2":
+            cf = self.cf(l)
+            nrows = int(np.count_nonzero((cf == 1) | (cf == -2)))   # the first-stage C points
+            rp = np.empty(nrows + 1, dtype=np.int32)
+            check(lib().hdk_amg_get_matrix(self.h, l, code, rp.ctypes.data, None, None))
+            cj = np.empty(max(int(rp[nrows]), 1), dtype=np.int32)
+            check(lib().hdk_amg_get_matrix(self.h, l, code, rp.ctypes.data, cj.ctypes.data, None))
+            return rp, cj[:int(rp[nrows])], np.ones(int(rp[nrows]))
         info = self.level_info(l)
         if which == "A":
             nrows, nnz = info["rows"], info["nnz_A"]

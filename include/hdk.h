@@ -137,6 +137,15 @@ typedef struct
     * [0, num_functions), read during the setup only; NULL = interleaved (global row % num_functions) */
    int            num_functions; /* 1 */
    const int32_t *dof_func;      /* NULL */
+   /* aggressive coarsening (hypre agg_num_levels ...): on levels l < agg_num_levels a second PMIS
+    * stage runs on the C points over the paths of length <= 2 (at least agg_num_paths of them), and
+    * P is multipass interpolation (agg_interp_type 4, the only type with a device kernel), each pass
+    * truncated by agg_trunc_factor / agg_max_nnz_row (0: no limit).  Needs num_functions == 1. */
+   int    agg_num_levels;   /* 0 */
+   int    agg_num_paths;    /* 1 */
+   int    agg_interp_type;  /* 4 = multipass */
+   int    agg_max_nnz_row;  /* 0 */
+   double agg_trunc_factor; /* 0 */
 } hdk_amg_params;
 
 void hdk_amg_default_params(hdk_amg_params *p);
@@ -152,7 +161,10 @@ int  hdk_amg_vcycle(hdk_amg *M, const double *f_d, double *u_d);
 int hdk_amg_num_levels(const hdk_amg *M);
 int hdk_amg_num_dist_levels(const hdk_amg *M); /* N > 1: leading levels that are row-distributed (the rest is replicated) */
 int hdk_amg_level_info(const hdk_amg *M, int level, int64_t *rows, int64_t *nnz_A, int64_t *nnz_P);
-/* which: 0 = A_l, 1 = P_l, 2 = R_l, 3 = S_l (pattern; val_h may be NULL) -- local diag block */
+/* which: 0 = A_l, 1 = P_l, 2 = R_l, 3 = S_l (pattern; val_h may be NULL) -- local diag block;
+ * 4 = S2_l, the second-stage strength of an aggressive level over its first-stage C points (pattern,
+ * amg_keep_debug only, like S_l).  col_h == NULL copies the row pointers alone (S2 can hold more
+ * entries than A_l, so a caller sizes the column buffer from them). */
 int hdk_amg_get_matrix(const hdk_amg *M, int level, int which, int32_t *rowptr_h,
                        int32_t *col_h, double *val_h);
 /* N > 1 (row-distributed setup), tunable amg_keep_debug set before the setup: this rank's rows of
