@@ -20,6 +20,10 @@ struct AmgLevel
    double    *u = nullptr, *f = nullptr, *t = nullptr;
    double    *gs1 = nullptr, *gs2 = nullptr; // two-stage GS: correction vectors of the inner steps
    DevCSR     L;            // strict lower triangle (two-stage GS only)
+   // Chebyshev smoothing (relax 16): D^{-1/2} (ones when unscaled), the sweep's scaled residual and the
+   // two alternating polynomial states; eigenvalue bounds (max, min) and coefficients c_0..c_{order-1}
+   double    *cheb_ds = nullptr, *cheb_r = nullptr, *cheb_v[2] = {nullptr, nullptr};
+   double     cheb_eig[2] = {0.0, 0.0}, cheb_c[4] = {0.0, 0.0, 0.0, 0.0};
    int        n = 0;
    // distributed setup, amg_keep_debug: my rows of P_l and A_l with GLOBAL columns in the serial
    // storage order (what the parity tests compare with the oracle, slab by slab)
@@ -90,5 +94,8 @@ int amg_cycle(hdk_amg_s *M, const double *f, double *u, bool zero_guess, int fin
 int exclusive_scan_int(const int *in, int *out, int n);       // hdk_csr.cu (hand-written reduce-then-scan)
 int exclusive_scan_i64(const int *in, int64_t *out, int n);
 int exclusive_scan_i64_i64(const int64_t *in, int64_t *out, int64_t n);
+// Chebyshev (hdk_spmv.cu): y = the epilogue of `mode` (SPMV_CHEB_*) applied to a finished row result
+// acc (A x, or b - A x for START / ONE), element-wise; the unfused form and the zero-guess start
+int cheb_epilogue_pass(int mode, int n, const double *acc, const SpmvArgs &a);
 bool amg_prefill_target(hdk_amg_s *M, double *z, double **buf, const double **d, double *w, const hdk_csr_s **reader = nullptr);
 } // namespace hdk

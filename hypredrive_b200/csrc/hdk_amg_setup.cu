@@ -2842,6 +2842,7 @@ void hdk_amg_default_params(hdk_amg_params *p)
    p->rand_seed = 2747; p->keep_transpose = 1; p->print_level = 0;
    p->num_functions = 1; p->dof_func = NULL;
    p->agg_num_levels = 0; p->agg_num_paths = 1; p->agg_interp_type = 4; p->agg_max_nnz_row = 0; p->agg_trunc_factor = 0.0;
+   p->cheby_order = 2; p->cheby_fraction = 0.3; p->cheby_eig_est = 10; p->cheby_variant = 0; p->cheby_scale = 1;
 }
 
 int hdk_amg_destroy(hdk_amg *M)
@@ -2858,6 +2859,7 @@ int hdk_amg_destroy(hdk_amg *M)
          if (L.l1_up != L.l1_down) dfree(L.l1_up);
          dfree(L.l1_down);
          dfree(L.u); dfree(L.f); dfree(L.t); dfree(L.gs1); dfree(L.gs2);
+         dfree(L.cheb_ds); dfree(L.cheb_r); dfree(L.cheb_v[0]); dfree(L.cheb_v[1]);
          for (int w = 0; w < 2; w++) { dfree(L.dbg_ip[w]); dfree(L.dbg_col[w]); dfree(L.dbg_val[w]); }
       }
       dfree(M->ge_inv); dfree(M->full_f); dfree(M->full_u);
@@ -2868,6 +2870,282 @@ int hdk_amg_destroy(hdk_amg *M)
    if (M->tail) hdk_amg_destroy(M->tail);
    delete M;
    return HDK_OK;
+}
+
+// =====================================================================================
+// Chebyshev smoothing (relax 16, hypre_ParCSRRelax_Cheby_Setup; rule in DESIGN.md section 4):
+// D^{-1/2}, eigenvalue bounds of C A (Gershgorin or CG-Lanczos), interval and coefficients
+// =====================================================================================
+constexpr int CHEB_RT = 256;
+// per row: ds = 1/sqrt|a_ii| (scaled) or 1, |a_ii|, and the Gershgorin bounds (|a_ii| +- R_i) [/ |a_ii|]
+// reduced per block to (max hi, max -lo, zero diagonal seen) in partials[3 b ..]
+__global__ void __launch_bounds__(CHEB_RT) k_cheb_rows(const int *rp, const int *col, const double *val, const int *orp,
+                                                       const double *oval, int n, int scale, double *ds, double *dabs,
+                                                       double *partials)
+{
+   __shared__ double sm[3][CHEB_RT];
+   double hi = -INFINITY, nlo = -INFINITY, bad = 0.0;
+   for (int i = blockIdx.x * CHEB_RT + threadIdx.x; i < n; i += gridDim.x * CHEB_RT)
+   {
+      double d = 0.0, R = 0.0;
+      for (int k = rp[i]; k < rp[i + 1]; k++)
+      {
+         if (col[k] == i) d = __dadd_rn(d, val[k]);
+         else R = __dadd_rn(R, fabs(val[k]));
+      }
+      if (orp) for (int k = orp[i]; k < orp[i + 1]; k++) R = __dadd_rn(R, fabs(oval[k]));
+      const double ad = fabs(d);
+      dabs[i] = ad;
+      if (scale && ad == 0.0) { bad = 1.0; ds[i] = 0.0; continue; }
+      ds[i] = scale ? __ddiv_rn(1.0, __dsqrt_rn(ad)) : 1.0;
+      const double h = scale ? __ddiv_rn(__dadd_rn(ad, R), ad) : __dadd_rn(ad, R);
+      const double l = scale ? __ddiv_rn(__dadd_rn(ad, -R), ad) : __dadd_rn(ad, -R);
+      hi  = fmax(hi, h);
+      nlo = fmax(nlo, -l);
+   }
+   sm[0][threadIdx.x] = hi; sm[1][threadIdx.x] = nlo; sm[2][threadIdx.x] = bad;
+   __syncthreads();
+   for (int o = CHEB_RT / 2; o > 0; o >>= 1)
+   {
+      if (threadIdx.x < o)
+         for (int q = 0; q < 3; q++) sm[q][threadIdx.x] = fmax(sm[q][threadIdx.x], sm[q][threadIdx.x + o]);
+      __syncthreads();
+   }
+   if (threadIdx.x < 3) partials[3 * blockIdx.x + threadIdx.x] = sm[threadIdx.x][0];
+}
+__global__ void k_cheb_rows_fold(const double *partials, int nb, double *out)
+{
+   if (threadIdx.x >= 3) return;
+   double m = -INFINITY;
+   for (int b = 0; b < nb; b++) m = fmax(m, partials[3 * b + threadIdx.x]);
+   out[threadIdx.x] = m;
+}
+
+// CG-Lanczos estimate (hypre_ParCSRMaxEigEstimateCG): preconditioned CG with C = D^{-1} (scaled) or I.
+// The scalars stay on the device in h[]: gamma (double-buffered by step parity), <s,p>, <r,z>, a stop
+// flag with the number of completed steps, and per step j: alpha_j at H_HIST + 2j, beta_{j+1} after it.
+enum { H_G = 0, H_SP = 2, H_GN = 3, H_STOP = 4, H_M = 5, H_HIST = 8 };
+__global__ void k_cheb_cg_init(const double *b, const double *dabs, int scale, int n, double *r, double *z, double *p)
+{
+   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+   {
+      const double zi = scale ? __ddiv_rn(b[i], dabs[i]) : b[i];
+      r[i] = b[i]; z[i] = zi; p[i] = zi;
+   }
+}
+// alpha_j = gamma_j / <s,p>; r -= alpha s; z = C r  (stop when <s,p> <= 0)
+__global__ void k_cheb_cg_r(double *h, int j, const double *s, const double *dabs, int scale, int n, double *r, double *z)
+{
+   if (h[H_STOP] != 0.0) return;
+   const double sp = h[H_SP];
+   const bool   t0 = blockIdx.x == 0 && threadIdx.x == 0;
+   if (!(sp > 0.0)) { if (t0) { h[H_STOP] = 1.0; h[H_M] = j; } return; }
+   const double alpha = __ddiv_rn(h[H_G + (j & 1)], sp);
+   if (t0) h[H_HIST + 2 * j] = alpha;
+   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+   {
+      const double ri = __dadd_rn(r[i], -__dmul_rn(alpha, s[i]));
+      r[i] = ri;
+      z[i] = scale ? __ddiv_rn(ri, dabs[i]) : ri;
+   }
+}
+// beta_{j+1} = <r,z> / gamma_j; p = z + beta p  (stop after this step when <r,z> <= 0)
+__global__ void k_cheb_cg_p(double *h, int j, const double *z, int n, double *p)
+{
+   if (h[H_STOP] != 0.0) return;
+   const double gn = h[H_GN];
+   const bool   t0 = blockIdx.x == 0 && threadIdx.x == 0;
+   if (!(gn > 0.0)) { if (t0) { h[H_STOP] = 1.0; h[H_M] = j + 1; } return; }
+   const double beta = __ddiv_rn(gn, h[H_G + (j & 1)]);
+   if (t0) { h[H_HIST + 2 * j + 1] = beta; h[H_G + ((j + 1) & 1)] = gn; }
+   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) p[i] = __dadd_rn(z[i], __dmul_rn(beta, p[i]));
+}
+
+// Eigenvalues of the symmetric tridiagonal matrix (d diagonal, e[1..n-1] sub-diagonal) by the implicit
+// QL iteration of EISPACK tql1 (hypre_LINPACKcgtql1); ascending in d.  -1: no convergence.
+static double cheb_pythag(double a, double b)
+{
+   double p = fmax(fabs(a), fabs(b));
+   if (p == 0.0) return 0.0;
+   double q = fmin(fabs(a), fabs(b)) / p;
+   return p * sqrt(1.0 + q * q);
+}
+static int cheb_tql1(int n, double *d, double *e)
+{
+   if (n == 1) return 0;
+   for (int i = 1; i < n; i++) e[i - 1] = e[i];
+   e[n - 1] = 0.0;
+   double f = 0.0, tst1 = 0.0;
+   for (int l = 0; l < n; l++)
+   {
+      int    it = 0, m;
+      double h = fabs(d[l]) + fabs(e[l]);
+      if (tst1 < h) tst1 = h;
+      for (m = l; m < n; m++)
+         if (tst1 + fabs(e[m]) == tst1) break;
+      if (m > l)
+      {
+         for (;;)
+         {
+            if (it++ == 30) return -1;
+            const int l1 = l + 1;
+            double    g = d[l];
+            double    p = (d[l1] - g) / (2.0 * e[l]);
+            double    r = cheb_pythag(p, 1.0);
+            double    sr = (p >= 0.0) ? fabs(r) : -fabs(r);
+            d[l]  = e[l] / (p + sr);
+            d[l1] = e[l] * (p + sr);
+            double dl1 = d[l1];
+            h = g - d[l];
+            for (int i = l1 + 1; i < n; i++) d[i] -= h;
+            f += h;
+            p = d[m];
+            double c = 1.0, c2 = c, c3 = c, el1 = e[l1], s = 0.0, s2 = 0.0;
+            for (int i = m - 1; i >= l; i--)
+            {
+               c3 = c2; c2 = c; s2 = s;
+               g = c * e[i];
+               h = c * p;
+               r = cheb_pythag(p, e[i]);
+               e[i + 1] = s * r;
+               s = e[i] / r;
+               c = p / r;
+               p = c * d[i] - s * g;
+               d[i + 1] = h + s * (c * g + s * d[i]);
+            }
+            p = -s * s2 * c3 * el1 * e[l] / dl1;
+            e[l] = s * p;
+            d[l] = c * p;
+            if (!(tst1 + fabs(e[l]) > tst1)) break;
+         }
+      }
+      double p = d[l] + f;
+      int    i = l;
+      for (; i > 0 && p < d[i - 1]; i--) d[i] = d[i - 1];
+      d[i] = p;
+   }
+   return 0;
+}
+
+// interval and monomial coefficients of s(t) = (1 - T_k((theta - t)/delta) / T_k(theta/delta)) / t
+static int cheb_coefs(double max_eig, double min_eig, double fraction, int order, double *c, int level)
+{
+   double upper, lower;
+   if (min_eig >= 0.0) { upper = 1.1 * max_eig; lower = (upper - min_eig) * fraction + min_eig; }
+   else if (max_eig <= 0.0) { upper = 1.1 * min_eig; lower = max_eig - (max_eig - upper) * fraction; }
+   else { const double mn = 0.0; upper = 1.1 * max_eig; lower = (upper - mn) * fraction + mn; }
+   const double theta = (upper + lower) / 2.0, delta = (upper - lower) / 2.0;
+   if (theta == 0.0 || !isfinite(theta) || !isfinite(delta))
+      return set_error(HDK_ERR_INVALID, "Chebyshev smoother on level %d: degenerate eigenvalue interval [%g, %g]", level, lower, upper);
+   const double t2 = theta * theta, d2 = delta * delta;
+   if (order == 1) c[0] = 1.0 / theta;
+   else if (order == 2)
+   {
+      const double den = d2 - 2.0 * t2;
+      c[0] = -4.0 * theta / den; c[1] = 2.0 / den;
+   }
+   else if (order == 3)
+   {
+      const double den = 4.0 * t2 * theta - 3.0 * d2 * theta;
+      c[0] = (12.0 * t2 - 3.0 * d2) / den; c[1] = -12.0 * theta / den; c[2] = 4.0 / den;
+   }
+   else
+   {
+      const double den = 8.0 * t2 * t2 - 8.0 * d2 * t2 + d2 * d2;
+      c[0] = (32.0 * t2 * theta - 16.0 * d2 * theta) / den; c[1] = -(48.0 * t2 - 8.0 * d2) / den;
+      c[2] = 32.0 * theta / den; c[3] = -8.0 / den;
+   }
+   for (int i = 0; i < order; i++)
+      if (!isfinite(c[i])) return set_error(HDK_ERR_INVALID, "Chebyshev smoother on level %d: coefficient %d is not finite", level, i);
+   return HDK_OK;
+}
+
+// everything a Chebyshev sweep on level l needs; dist: the level is row-distributed over the ranks
+static int cheby_setup_level(AmgLevel &L, const hdk_amg_params *prm, int level, bool dist)
+{
+   const hdk_csr_s &A = *L.A;
+   const int        n = L.n, k = prm->cheby_eig_est, scale = prm->cheby_scale;
+   HDK_TRY(dalloc(&L.cheb_ds, (size_t)n + 8));
+   HDK_TRY(dalloc(&L.cheb_r, (size_t)n + 8));
+   HDK_TRY(dalloc(&L.cheb_v[0], (size_t)n + 8));
+   HDK_TRY(dalloc(&L.cheb_v[1], (size_t)n + 8));
+   double *dabs, *h;
+   HDK_TRY(dalloc(&dabs, (size_t)n + 8));
+   HDK_TRY(dalloc(&h, (size_t)H_HIST + 2 * (size_t)k + 8));
+   HDK_CUDA(cudaMemsetAsync(h, 0, sizeof(double) * ((size_t)H_HIST + 2 * (size_t)k + 8), g.stream));
+   int nb = cdiv(n, CHEB_RT);
+   if (nb > g.sm_count * 4) nb = g.sm_count * 4;
+   if (nb < 1) nb = 1;
+   const bool    offd = A.offd.nnz > 0;
+   k_cheb_rows<<<nb, CHEB_RT, 0, g.stream>>>(A.diag.rowptr, A.diag.col, A.diag.val, offd ? A.offd.rowptr : nullptr,
+                                             offd ? A.offd.val : nullptr, n, scale, L.cheb_ds, dabs, g.partials);
+   HDK_LAUNCH_CHECK();
+   k_cheb_rows_fold<<<1, 32, 0, g.stream>>>(g.partials, nb, h + H_HIST - 3); // (h[5..7]: free until the CG starts)
+   HDK_LAUNCH_CHECK();
+   if (dist) HDK_TRY(allreduce_max_dev(h + H_HIST - 3, 3));
+   double gb[3];
+   HDK_CUDA(cudaMemcpyAsync(gb, h + H_HIST - 3, sizeof(gb), cudaMemcpyDeviceToHost, g.stream));
+   HDK_CUDA(cudaStreamSynchronize(g.stream));
+   int rc = HDK_OK;
+   if (gb[2] != 0.0) rc = set_error(HDK_ERR_INVALID, "Chebyshev smoother on level %d: a row has a zero diagonal (the scaling D^{-1/2} needs a_ii != 0)", level);
+   double max_eig = gb[0], min_eig = -gb[1];
+   if (rc == HDK_OK && k > 0)
+   {
+      HDK_CUDA(cudaMemsetAsync(h, 0, sizeof(double) * H_HIST, g.stream));
+      double *r = L.cheb_r, *z = L.cheb_v[0], *p = L.cheb_v[1], *s = L.t;
+      const int grid = nb;
+      HDK_TRY(hdk_vec_random(s, n, A.row_start, 1));
+      k_cheb_cg_init<<<grid, CHEB_RT, 0, g.stream>>>(s, dabs, scale, n, r, z, p);
+      HDK_LAUNCH_CHECK();
+      HDK_TRY(vec_dot_dev(r, z, n, FIN_STORE, h + H_G));
+      if (dist) HDK_TRY(allreduce_dev(h + H_G, 1));
+      for (int j = 0; j < k; j++)
+      {
+         SpmvArgs a;
+         a.x = p; a.y = s;
+         HDK_TRY(parcsr_matvec(A, SPMV_SET, a));
+         HDK_TRY(vec_dot_dev(s, p, n, FIN_STORE, h + H_SP));
+         if (dist) HDK_TRY(allreduce_dev(h + H_SP, 1));
+         k_cheb_cg_r<<<grid, CHEB_RT, 0, g.stream>>>(h, j, s, dabs, scale, n, r, z);
+         HDK_LAUNCH_CHECK();
+         HDK_TRY(vec_dot_dev(r, z, n, FIN_STORE, h + H_GN));
+         if (dist) HDK_TRY(allreduce_dev(h + H_GN, 1));
+         k_cheb_cg_p<<<grid, CHEB_RT, 0, g.stream>>>(h, j, z, n, p);
+         HDK_LAUNCH_CHECK();
+      }
+      std::vector<double> hh((size_t)H_HIST + 2 * (size_t)k);
+      HDK_CUDA(cudaMemcpyAsync(hh.data(), h, sizeof(double) * hh.size(), cudaMemcpyDeviceToHost, g.stream));
+      HDK_CUDA(cudaStreamSynchronize(g.stream));
+      const int m = hh[H_STOP] != 0.0 ? (int)hh[H_M] : k;
+      if (m < 1) rc = set_error(HDK_ERR_INVALID, "Chebyshev smoother on level %d: the CG eigenvalue estimate broke down at its first step", level);
+      else
+      {
+         // Lanczos tridiagonal: T_jj = 1/alpha_j + beta_j/alpha_{j-1}, T_{j,j+1} = sqrt(beta_{j+1})/alpha_j
+         std::vector<double> d((size_t)m), e((size_t)m, 0.0);
+         const double       *al = &hh[H_HIST];
+         for (int j = 0; j < m; j++)
+         {
+            d[(size_t)j] = (j == 0) ? 1.0 / al[0] : 1.0 / al[2 * j] + al[2 * j - 1] / al[2 * j - 2];
+            if (j > 0) e[(size_t)j] = sqrt(al[2 * j - 1]) / al[2 * j - 2];
+         }
+         if (cheb_tql1(m, d.data(), e.data()) != 0) rc = set_error(HDK_ERR_INVALID, "Chebyshev smoother on level %d: no convergence of the tridiagonal eigenvalue iteration", level);
+         max_eig = d[(size_t)m - 1]; min_eig = d[0];
+      }
+   }
+   dfree(dabs); dfree(h);
+   if (rc != HDK_OK) return rc;
+   L.cheb_eig[0] = max_eig; L.cheb_eig[1] = min_eig;
+   return cheb_coefs(max_eig, min_eig, prm->cheby_fraction, prm->cheby_order, L.cheb_c, level);
+}
+
+// algorithmic bytes of one Chebyshev sweep (hdk_time_kernel 9): order k reads A k times; START and FIN
+// move five vectors, STEP four; from a zero guess the first pass is element-wise and FIN reads no u_old
+static double cheb_sweep_bytes(int order, double n, double nnz, bool zero_guess)
+{
+   const double pass = 12.0 * nnz + 4.0 * (n + 1);
+   if (order == 1) return zero_guess ? 24.0 * n : pass + 32.0 * n;
+   if (zero_guess) return 32.0 * n + (order - 1) * pass + (order - 2) * 32.0 * n + 32.0 * n;
+   return order * pass + 40.0 * n + (order - 2) * 32.0 * n + 40.0 * n;
 }
 
 // per-level solve data: smoother diagonals, work vectors, (two-stage GS) lower triangles, and the
@@ -2893,17 +3171,27 @@ int finalize_levels(hdk_amg_s *M, const hdk_amg_params *prm, int64_t live_max_ro
       bool tsgs = (prm->relax_down == 11 || prm->relax_down == 12 || prm->relax_up == 11 || prm->relax_up == 12);
       if (tsgs && (rc = build_lower(L.A->diag, L.L))) break;
       if (tsgs && ((rc = dalloc(&L.gs1, (size_t)n + 8)) || (rc = dalloc(&L.gs2, (size_t)n + 8)))) break;
+      // Chebyshev data where a sweep runs: smoothing levels for down / up, the coarsest for the coarse solve
+      // (relax 16 builds no dense inverse); levels of a hierarchy with a replicated tail are row-distributed
+      const bool cheb = L.P ? (prm->relax_down == 16 || prm->relax_up == 16) : (prm->relax_coarse == 16 && !M->tail);
+      if (cheb && (rc = cheby_setup_level(L, prm, l, M->tail != nullptr && g.nranks > 1))) break;
       // algorithmic bytes of one V-cycle (DESIGN.md): zero-guess pre-smooth 24n, residual,
       // restriction, prolongation, post-smooth
       double nnzA = (double)L.A->diag.nnz + L.A->offd.nnz;
       if (L.P)
       {
          double nnzP = (double)L.P->diag.nnz + L.P->offd.nnz, ncl = (double)L.P->diag.ncols;
-         bytes += 24.0 * n;                                       // u = w f / d
+         bytes += prm->relax_down == 16 ? cheb_sweep_bytes(prm->cheby_order, n, nnzA, true) : 24.0 * n; // u = w f / d
          bytes += 12.0 * nnzA + 4.0 * (n + 1) + 24.0 * n;         // r = f - A u
          bytes += 12.0 * nnzP + 4.0 * (ncl + 1) + 8.0 * n + 8.0 * ncl; // f_c = R r
          bytes += 12.0 * nnzP + 4.0 * (n + 1) + 16.0 * n + 8.0 * ncl;  // u += P e
-         bytes += 12.0 * nnzA + 4.0 * (n + 1) + 32.0 * n;         // post-smooth
+         bytes += prm->relax_up == 16 ? cheb_sweep_bytes(prm->cheby_order, n, nnzA, false)
+                                      : 12.0 * nnzA + 4.0 * (n + 1) + 32.0 * n; // post-smooth
+      }
+      else if (prm->relax_coarse == 16)
+      {
+         const int sw = prm->sweeps_coarse < 1 ? 1 : prm->sweeps_coarse;
+         bytes += cheb_sweep_bytes(prm->cheby_order, n, nnzA, true) + (sw - 1) * cheb_sweep_bytes(prm->cheby_order, n, nnzA, false);
       }
       else bytes += 8.0 * (double)n * n + 16.0 * n;
    }
@@ -3298,6 +3586,15 @@ int hdk_amg_setup(const hdk_csr *A0, const hdk_amg_params *prm, hdk_amg **out)
       if (prm->num_functions > 1)
          return set_error(HDK_ERR_UNSUPPORTED, "aggressive coarsening with num_functions = %d has no device setup", prm->num_functions);
    }
+   if (prm->relax_down == 16 || prm->relax_up == 16 || prm->relax_coarse == 16)
+   {
+      if (prm->cheby_order < 1 || prm->cheby_order > 4) return set_error(HDK_ERR_INVALID, "cheby_order must be in 1..4 (got %d)", prm->cheby_order);
+      if (!(prm->cheby_fraction > 0.0 && prm->cheby_fraction <= 1.0)) return set_error(HDK_ERR_INVALID, "cheby_fraction must be in (0, 1] (got %g)", prm->cheby_fraction);
+      if (prm->cheby_eig_est < 0) return set_error(HDK_ERR_INVALID, "cheby_eig_est must be at least 0 (got %d)", prm->cheby_eig_est);
+      if (prm->cheby_variant == 1) return set_error(HDK_ERR_UNSUPPORTED, "cheby_variant 1 has no device implementation (use 0)");
+      if (prm->cheby_variant != 0) return set_error(HDK_ERR_INVALID, "cheby_variant must be 0 or 1 (got %d)", prm->cheby_variant);
+      if (prm->cheby_scale != 0 && prm->cheby_scale != 1) return set_error(HDK_ERR_INVALID, "cheby_scale must be 0 or 1 (got %d)", prm->cheby_scale);
+   }
    g_timing = getenv("HDK_SETUP_TIMING") && atoi(getenv("HDK_SETUP_TIMING")) == 1;
    // row-distributed setup (hdk_amg_dist.cu); HDK_SETUP_REPLICATED=1 selects the round-1 scheme that
    // rebuilds the global hierarchy on every rank (kept for comparison)
@@ -3385,6 +3682,20 @@ int hdk_amg_get_l1(const hdk_amg *M, int level, double *l1_h)
    M = resolve_level(M, level);
    if (!M || level < 0 || level >= M->nlev) return set_error(HDK_ERR_INVALID, "level out of range");
    return get_level_array(M, level, M->lev[(size_t)level].l1_down, sizeof(double) * (size_t)M->lev[(size_t)level].n, l1_h);
+}
+
+int hdk_amg_get_cheby(const hdk_amg *M, int level, double *eig_h, double *coefs_h, double *ds_h)
+{
+   HDK_TRY(require_init());
+   const int asked = level;
+   M = resolve_level(M, level);
+   if (!M || level < 0 || level >= M->nlev) return set_error(HDK_ERR_INVALID, "level out of range");
+   const AmgLevel &L = M->lev[(size_t)level];
+   if (!L.cheb_ds) return set_error(HDK_ERR_INVALID, "level %d has no Chebyshev data (no sweep of relaxation type 16 runs there)", asked);
+   if (eig_h) { eig_h[0] = L.cheb_eig[0]; eig_h[1] = L.cheb_eig[1]; }
+   if (coefs_h) for (int i = 0; i < M->prm.cheby_order; i++) coefs_h[i] = L.cheb_c[i];
+   if (ds_h) return hdk_copy_d2h(ds_h, L.cheb_ds, sizeof(double) * (size_t)L.n);
+   return HDK_OK;
 }
 
 int hdk_amg_strength(const hdk_csr *A, double theta, double max_row_sum, int64_t *nnz_S, int32_t **rowptr_d, int32_t **col_d)

@@ -23,11 +23,92 @@ __global__ void __launch_bounds__(256) k_dense_apply(const double *__restrict__ 
 
 static bool is_jacobi(int t) { return t == 18 || t == 7 || t == 0; }
 
+// One Chebyshev sweep (relax 16, hypre_ParCSRRelax_Cheby_Solve, scaled form; DESIGN.md section 4):
+//   r = ds (f - A u);  v = c_{k-1} r;  v = c_i r + ds (A (ds v)) for i = k-2..0;  out = u + ds v
+// The passes carry w = ds v, so every pass is one product with a fused epilogue: START (r and w),
+// STEP (w), FIN (out, optionally with the fused dot <f, out>); order 1 is the single pass ONE.
+// in == nullptr: zero initial guess, the first pass is element-wise (f - A 0 = f).  Levels whose
+// off-rank part is added by a correction kernel run each pass as a plain product + element-wise epilogue.
+static int cheby_sweep(hdk_amg_s *M, int l, const double *f, const double *in, double *out, int fin, double *fin_out,
+                       const hdk_csr_s *export_to = nullptr)
+{
+   AmgLevel &L = M->lev[(size_t)l];
+   if (!L.cheb_ds) return set_error(HDK_ERR_INVALID, "level %d has no Chebyshev data", l);
+   const int     k = M->prm.cheby_order, n = L.n;
+   const bool    fused = parcsr_single_kernel(*L.A);
+   const double *c = L.cheb_c;
+   SpmvArgs      a;
+   a.d = L.cheb_ds;
+   if (k == 1)
+   {
+      a.b = f; a.alpha = c[0]; a.uo = in; a.y = out;
+      if (!in) HDK_TRY(cheb_epilogue_pass(SPMV_CHEB_ONE, n, f, a));
+      else if (fused)
+      {
+         a.x = in; a.export_to = export_to;
+         if (fin != FIN_NONE) { a.dotv = f; a.fin = fin; a.fin_out = fin_out; fin = FIN_NONE; }
+         HDK_TRY(parcsr_matvec(*L.A, SPMV_CHEB_ONE, a));
+      }
+      else
+      {
+         SpmvArgs rr;
+         rr.x = in; rr.b = f; rr.y = L.cheb_r;
+         HDK_TRY(parcsr_matvec(*L.A, SPMV_RESIDUAL, rr));
+         HDK_TRY(cheb_epilogue_pass(SPMV_CHEB_ONE, n, L.cheb_r, a));
+      }
+   }
+   else
+   {
+      double *cur = L.cheb_v[0], *nxt = L.cheb_v[1];
+      // START: r = ds (f - A u), w = ds (c_{k-1} r)
+      a.b = f; a.alpha = c[k - 1]; a.y = cur; a.y2 = L.cheb_r;
+      if (!in) HDK_TRY(cheb_epilogue_pass(SPMV_CHEB_START, n, f, a));
+      else if (fused)
+      {
+         a.x = in; a.export_to = L.A;
+         HDK_TRY(parcsr_matvec(*L.A, SPMV_CHEB_START, a));
+      }
+      else
+      {
+         SpmvArgs rr;
+         rr.x = in; rr.b = f; rr.y = nxt;
+         HDK_TRY(parcsr_matvec(*L.A, SPMV_RESIDUAL, rr));
+         HDK_TRY(cheb_epilogue_pass(SPMV_CHEB_START, n, nxt, a));
+      }
+      for (int i = k - 2; i >= 0; i--)
+      {
+         // STEP: w' = ds (c_i r + ds (A w)); the last one (i = 0) is FIN: out = u + ds (c_0 r + ds (A w))
+         const int mode = (i == 0) ? SPMV_CHEB_FIN : SPMV_CHEB_STEP;
+         SpmvArgs  b2;
+         b2.d = L.cheb_ds; b2.b = L.cheb_r; b2.alpha = c[i];
+         b2.y = (i == 0) ? out : nxt;
+         b2.uo = in;
+         if (fused)
+         {
+            b2.x = cur; b2.export_to = (i == 0) ? export_to : L.A;
+            if (i == 0 && fin != FIN_NONE) { b2.dotv = f; b2.fin = fin; b2.fin_out = fin_out; fin = FIN_NONE; }
+            HDK_TRY(parcsr_matvec(*L.A, mode, b2));
+         }
+         else
+         {
+            SpmvArgs pr;
+            pr.x = cur; pr.y = b2.y;
+            HDK_TRY(parcsr_matvec(*L.A, SPMV_SET, pr));
+            HDK_TRY(cheb_epilogue_pass(mode, n, b2.y, b2));
+         }
+         std::swap(cur, nxt);
+      }
+   }
+   if (fin != FIN_NONE) HDK_TRY(vec_dot_dev(f, out, n, fin, fin_out));
+   return HDK_OK;
+}
+
 // one smoothing sweep u_new = S(u_old); result written to `out` (out != in)
 // export_to: the matrix whose product reads `out` next (its halo is filled by this sweep's kernel)
 static int relax_sweep(hdk_amg_s *M, int l, int type, const double *l1, const double *f, const double *in,
                        double *out, int fin, double *fin_out, const hdk_csr_s *export_to = nullptr)
 {
+   if (type == 16) return cheby_sweep(M, l, f, in, out, fin, fin_out, export_to);
    AmgLevel &L = M->lev[(size_t)l];
    SpmvArgs  a;
    a.x = in; a.y = out; a.b = f; a.d = l1; a.w = M->prm.relax_weight;
@@ -89,7 +170,7 @@ static int relax_sweep(hdk_amg_s *M, int l, int type, const double *l1, const do
       if (fin != FIN_NONE) HDK_TRY(vec_dot_dev(f, out, L.n, fin, fin_out));
       return HDK_OK;
    }
-   return set_error(HDK_ERR_UNSUPPORTED, "relaxation type %d has no device kernel (use 18, 7, 0, 11 or 12)", type);
+   return set_error(HDK_ERR_UNSUPPORTED, "relaxation type %d has no device kernel (use 18, 7, 0, 11, 12 or 16)", type);
 }
 
 static int coarse_solve(hdk_amg_s *M, int l, const double *f, double *u, double *alt, bool zero_guess, double **result)
@@ -114,8 +195,12 @@ static int coarse_solve(hdk_amg_s *M, int l, const double *f, double *u, double 
       }
       else
       {
-         if (s == 0 && zero_guess) HDK_TRY(vec_fill(cur, 0.0, L.n));
-         HDK_TRY(relax_sweep(M, l, type, L.l1_down, f, cur, oth, FIN_NONE, nullptr));
+         if (s == 0 && zero_guess && type == 16) HDK_TRY(cheby_sweep(M, l, f, nullptr, oth, FIN_NONE, nullptr));
+         else
+         {
+            if (s == 0 && zero_guess) HDK_TRY(vec_fill(cur, 0.0, L.n));
+            HDK_TRY(relax_sweep(M, l, type, L.l1_down, f, cur, oth, FIN_NONE, nullptr));
+         }
          double *tmp = cur; cur = oth; oth = tmp;
       }
    }
@@ -154,7 +239,8 @@ static int first_graph_level(hdk_amg_s *M, int l0)
    const int64_t rows = tune_graph_rows();
    if (rows <= 0) return -1;
    const hdk_amg_params &p = M->prm;
-   if (!is_jacobi(p.relax_down) || !is_jacobi(p.relax_up)) return -1; // (two-stage GS may allocate scratch)
+   // (two-stage GS may allocate scratch; Chebyshev sweeps use preallocated buffers only)
+   if (!(is_jacobi(p.relax_down) || p.relax_down == 16) || !(is_jacobi(p.relax_up) || p.relax_up == 16)) return -1;
    for (int l = l0; l < M->nlev; l++)
       if (M->lev[(size_t)l].n <= rows) return l;
    return -1;
@@ -284,8 +370,13 @@ static int amg_cycle_impl(hdk_amg_s *M, const double *f0, double *u0, bool zero_
          else
          {
             tl_mark(l, 10);
-            if (s == 0 && zg) HDK_TRY(vec_fill(cur[(size_t)l], 0.0, L.n));
-            HDK_TRY(relax_sweep(M, l, p.relax_down, L.l1_down, rhs[(size_t)l], cur[(size_t)l], alt[(size_t)l], FIN_NONE, nullptr, L.A));
+            if (s == 0 && zg && p.relax_down == 16) // Chebyshev from a zero guess: no fill, no residual product
+               HDK_TRY(cheby_sweep(M, l, rhs[(size_t)l], nullptr, alt[(size_t)l], FIN_NONE, nullptr, L.A));
+            else
+            {
+               if (s == 0 && zg) HDK_TRY(vec_fill(cur[(size_t)l], 0.0, L.n));
+               HDK_TRY(relax_sweep(M, l, p.relax_down, L.l1_down, rhs[(size_t)l], cur[(size_t)l], alt[(size_t)l], FIN_NONE, nullptr, L.A));
+            }
             std::swap(cur[(size_t)l], alt[(size_t)l]);
          }
       }
@@ -482,6 +573,17 @@ int hdk_time_kernel(const hdk_csr *A, hdk_amg *M, int kernel, int reps, double *
                   rc = relax_sweep(M, 0, type, M->lev[0].l1_down, b, x, y, FIN_NONE, nullptr);
                   // stage 1 reads A, u, f, d and writes r, u+r; every inner step reads L, r, d, u and writes u (and r)
                   by = 12.0 * nnz + 4.0 * (n + 1) + 40.0 * n + (type == 11 ? 1 : 2) * (12.0 * nnzL + 4.0 * (n + 1) + 32.0 * n) + (type == 12 ? 8.0 * n : 0.0);
+               }
+               break;
+            case 9: // one Chebyshev sweep on the fine level (hierarchy set up with relaxation 16)
+               if (!M || M->nlev < 1 || !M->lev[0].cheb_ds) rc = set_error(HDK_ERR_INVALID, "Chebyshev timing needs a hierarchy whose fine level smooths with relaxation 16");
+               else
+               {
+                  const int    k = M->prm.cheby_order;
+                  const double pass = 12.0 * nnz + 4.0 * (n + 1);
+                  rc = cheby_sweep(M, 0, b, x, y, FIN_NONE, nullptr);
+                  // START reads u, f, ds and writes r, w; each STEP reads w, r, ds and writes w; FIN also reads u_old
+                  by = (k == 1) ? pass + 32.0 * n : k * pass + 40.0 * n + (k - 2) * 32.0 * n + 40.0 * n;
                }
                break;
             case 7: rc = halo_exchange_begin(*A, x); by = 8.0 * A->halo.n_send; break; // the halo exchange alone (N > 1)

@@ -128,7 +128,12 @@ enum SpmvMode
    SPMV_JACOBI_R = 5, // y = w*(b - A x)/d  (two-stage GS first stage)
    SPMV_SET_DIV = 6,  // y = A x ; y2 = w*y/d  (restriction fused with the next level's first l1-Jacobi sweep)
    SPMV_JACOBI2 = 7,  // y2 = w*(b - A x)/d ; y = x + y2   (two-stage GS, first stage: correction AND updated iterate)
-   SPMV_GS_STEP = 8   // t = (A x)/d ; y2 = t ; y = y + alpha*t   (two-stage GS inner step on the strict lower triangle)
+   SPMV_GS_STEP = 8,  // t = (A x)/d ; y2 = t ; y = y + alpha*t   (two-stage GS inner step on the strict lower triangle)
+   // Chebyshev sweep (relax 16), d = ds = |a_ii|^{-1/2}, alpha = the polynomial coefficient c, b = f or r
+   SPMV_CHEB_START = 10, // y2 = r = d (b - A x) ; y = d (c r)                   (first pass of an order >= 2 sweep)
+   SPMV_CHEB_STEP = 11,  // y = d (c b + d (A x))                                (b = r)
+   SPMV_CHEB_FIN = 12,   // y = uo + d (c b + d (A x))                           (b = r; uo = u_old, nullptr = 0)
+   SPMV_CHEB_ONE = 13    // y = uo + d (c (d (b - A x)))                         (order 1: the whole sweep)
 };
 
 // what the last block does with a fused dot product
@@ -160,6 +165,7 @@ struct SpmvArgs
    const double *xo = nullptr;  // halo part of x (offd block), appended columns
    double       *y2 = nullptr;  // second output of SPMV_SET_DIV
    double        w = 1.0, alpha = 1.0, beta = 0.0;
+   const double *uo = nullptr;  // iterate the Chebyshev finish adds to (SPMV_CHEB_FIN / _ONE; nullptr: zero)
    // fused dot: sum_i dotv[i]*y_new[i]  (dotv may alias x or b)
    const double *dotv = nullptr;
    int           fin = FIN_NONE;

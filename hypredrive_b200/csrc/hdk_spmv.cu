@@ -103,6 +103,7 @@ struct SpmvDev
    // halo of the NEXT product filled by this kernel (see HaloExport); exp_y2: the exported vector is y2
    HaloExport    exp;
    int           exp_y2;
+   const double *uo; // Chebyshev finish: the iterate the correction is added to (nullptr: zero)
 };
 
 // ---- PTX helpers: mbarrier + 1-D bulk tensor-memory-accelerator copies -------------------
@@ -158,6 +159,13 @@ __device__ __forceinline__ double store_out(const SpmvDev &a, int r, double v, d
       y2 = (dd != 0.0) ? __ddiv_rn(__dmul_rn(a.w, v), dd) : 0.0;
       a.y2[r] = y2;
    }
+   else if (MODE == SPMV_CHEB_START)
+   {
+      // v = r = ds (f - A u): kept for the later passes; y = ds (c r) is what the next product gathers
+      y2 = v;
+      a.y2[r] = y2;
+      yn = __dmul_rn(dd, __dmul_rn(a.alpha, v));
+   }
    a.y[r] = yn;
    // (compiled only into the multi-rank sliced-ELL variants: the plain kernels keep their 32 registers)
    if (EXP && a.exp.seq) nexp += export_row(a.exp, r, a.exp_y2 ? y2 : yn);
@@ -189,6 +197,26 @@ struct RowOps
    double b, d, xo, yo, dv;
 };
 
+// Chebyshev epilogues (relax 16), every product and sum rounded separately in the order of the
+// polynomial loop (DESIGN.md section 4): o.d = ds, o.b = f (START, ONE: acc is already f - A u) or the
+// scaled residual r (STEP, FIN: acc = A w), o.yo = u_old, alpha = the coefficient of this pass
+template <int MODE>
+__device__ __forceinline__ double cheb_epilogue(const SpmvDev &a, const RowOps &o, double acc)
+{
+   if (MODE == SPMV_CHEB_START) return __dmul_rn(o.d, acc);
+   if (MODE == SPMV_CHEB_ONE) return __dadd_rn(o.yo, __dmul_rn(o.d, __dmul_rn(a.alpha, __dmul_rn(o.d, acc))));
+   const double v = __dadd_rn(__dmul_rn(a.alpha, o.b), __dmul_rn(o.d, acc));
+   if (MODE == SPMV_CHEB_STEP) return __dmul_rn(o.d, v);
+   return __dadd_rn(o.yo, __dmul_rn(o.d, v));
+}
+template <int MODE>
+__device__ __forceinline__ void cheb_load(const SpmvDev &a, int r, RowOps &o)
+{
+   o.b = a.b[r];
+   o.d = a.d[r];
+   if (MODE == SPMV_CHEB_FIN || MODE == SPMV_CHEB_ONE) o.yo = a.uo ? a.uo[r] : 0.0;
+}
+
 template <int MODE, bool DOT>
 __device__ __forceinline__ void row_load(const SpmvDev &a, int r, int ka, RowOps &o)
 {
@@ -198,6 +226,7 @@ __device__ __forceinline__ void row_load(const SpmvDev &a, int r, int ka, RowOps
    if (MODE == SPMV_JACOBI || MODE == SPMV_JACOBI_R || MODE == SPMV_SET_DIV || MODE == SPMV_JACOBI2 || MODE == SPMV_GS_STEP) o.d = a.d[r];
    if (MODE == SPMV_JACOBI || MODE == SPMV_JACOBI2) o.xo = a.x[r];
    if (MODE == SPMV_ADD || MODE == SPMV_AXPBY) o.yo = a.y[r];
+   if (MODE >= SPMV_CHEB_START) cheb_load<MODE>(a, r, o);
    if (DOT) o.dv = a.dotv[r];
 }
 
@@ -205,7 +234,8 @@ __device__ __forceinline__ void row_load(const SpmvDev &a, int r, int ka, RowOps
 template <int MODE>
 __device__ __forceinline__ double row_compute(const SpmvDev &a, const RowOps &o, const double *vs, const int *cs)
 {
-   constexpr bool SUB = (MODE == SPMV_RESIDUAL || MODE == SPMV_JACOBI || MODE == SPMV_JACOBI_R || MODE == SPMV_JACOBI2);
+   constexpr bool SUB = (MODE == SPMV_RESIDUAL || MODE == SPMV_JACOBI || MODE == SPMV_JACOBI_R || MODE == SPMV_JACOBI2 ||
+                         MODE == SPMV_CHEB_START || MODE == SPMV_CHEB_ONE);
    double acc = SUB ? o.b : ((MODE == SPMV_ADD) ? o.yo : 0.0);
    int    k = o.s;
    // groups of four: issue the gathers together, then accumulate in order
@@ -228,6 +258,7 @@ __device__ __forceinline__ double row_compute(const SpmvDev &a, const RowOps &o,
       if (k + 1 < o.e) { double p1 = __dmul_rn(vs[k + 1], x1); acc = __dadd_rn(acc, SUB ? -p1 : p1); }
       if (k + 2 < o.e) { double p2 = __dmul_rn(vs[k + 2], x2); acc = __dadd_rn(acc, SUB ? -p2 : p2); }
    }
+   if (MODE >= SPMV_CHEB_START) return cheb_epilogue<MODE>(a, o, acc);
    if (MODE == SPMV_SET || MODE == SPMV_SET_DIV || MODE == SPMV_ADD || MODE == SPMV_RESIDUAL || MODE == SPMV_GS_STEP) return acc;
    if (MODE == SPMV_AXPBY)
       return (a.beta == 0.0) ? __dmul_rn(a.alpha, acc) : __dadd_rn(__dmul_rn(a.alpha, acc), __dmul_rn(a.beta, o.yo));
@@ -260,6 +291,8 @@ __device__ __forceinline__ double row_partial(const SpmvDev &a, int k, int e, co
 template <int MODE>
 __device__ __forceinline__ double row_finish(const SpmvDev &a, const RowOps &o, double total)
 {
+   if (MODE >= SPMV_CHEB_START)
+      return cheb_epilogue<MODE>(a, o, (MODE == SPMV_CHEB_START || MODE == SPMV_CHEB_ONE) ? __dadd_rn(o.b, -total) : total);
    if (MODE == SPMV_SET || MODE == SPMV_SET_DIV || MODE == SPMV_GS_STEP) return total;
    if (MODE == SPMV_ADD) return __dadd_rn(o.yo, total);
    if (MODE == SPMV_AXPBY)
@@ -425,6 +458,7 @@ constexpr int SELL_OFFD_BIT = 32; // sl_meta = len << 6 | row has off-rank entri
 template <int MODE>
 __device__ __forceinline__ double row_epilogue(const SpmvDev &a, const RowOps &o, double acc)
 {
+   if (MODE >= SPMV_CHEB_START) return cheb_epilogue<MODE>(a, o, acc);
    if (MODE == SPMV_SET || MODE == SPMV_SET_DIV || MODE == SPMV_ADD || MODE == SPMV_RESIDUAL || MODE == SPMV_GS_STEP) return acc;
    if (MODE == SPMV_AXPBY)
       return (a.beta == 0.0) ? __dmul_rn(a.alpha, acc) : __dadd_rn(__dmul_rn(a.alpha, acc), __dmul_rn(a.beta, o.yo));
@@ -460,7 +494,8 @@ __device__ __forceinline__ void sell_body(const SpmvDev &a)
 #ifdef HDK_XHINT
    const uint64_t xpol = x_policy();
 #endif
-   constexpr bool SUB  = (MODE == SPMV_RESIDUAL || MODE == SPMV_JACOBI || MODE == SPMV_JACOBI_R || MODE == SPMV_JACOBI2);
+   constexpr bool SUB  = (MODE == SPMV_RESIDUAL || MODE == SPMV_JACOBI || MODE == SPMV_JACOBI_R || MODE == SPMV_JACOBI2 ||
+                          MODE == SPMV_CHEB_START || MODE == SPMV_CHEB_ONE);
    constexpr bool DIAG = (MODE == SPMV_JACOBI || MODE == SPMV_JACOBI_R || MODE == SPMV_SET_DIV || MODE == SPMV_JACOBI2 || MODE == SPMV_GS_STEP);
    constexpr bool XOLD = (MODE == SPMV_JACOBI || MODE == SPMV_JACOBI2);
    __shared__ double red[SELL_T / 32];
@@ -484,8 +519,11 @@ __device__ __forceinline__ void sell_body(const SpmvDev &a)
       // (which operands are fetched before and which after the streaming loop is chosen by the
       // register count ptxas ends up with: 32 = 8 CTAs per SM, 33-40 = 6, 41-48 = 5)
       constexpr bool LATE = DOT; // fused-dot variants: smoother operands after the loop as well
+      // Chebyshev: the residual passes (START, ONE) fetch like the Jacobi modes, the others after the loop
+      constexpr bool CHEB_EARLY = MODE >= SPMV_CHEB_START && SUB && !LATE;
       if (valid)
       {
+         if (CHEB_EARLY) cheb_load<MODE>(a, r, o);
          if (SUB) o.b = a.b[r];
          if (!LATE && DIAG) o.d = a.d[r];
          if (!LATE && XOLD) o.xo = a.x[r];
@@ -537,6 +575,7 @@ __device__ __forceinline__ void sell_body(const SpmvDev &a)
       {
          if (LATE && DIAG) o.d = a.d[r];
          if (LATE && XOLD) o.xo = a.x[r];
+         if (MODE >= SPMV_CHEB_START && !CHEB_EARLY) cheb_load<MODE>(a, r, o);
          if (DOT) o.dv = a.dotv[r];
          // y += A x: y is read only now (live across the loop it costs 10 registers = 3 CTAs per SM),
          // so the sum is y + (a_0 x_0 + a_1 x_1 + ...) -- rounding-level difference to the CSR-order sum
@@ -667,7 +706,15 @@ __global__ void __launch_bounds__(ST) k_spmv_vector(SpmvDev a)
       double acc = 0.0;
       for (int k = s + lane; k < e; k += 32) acc += __ldg(a.val + k) * __ldg(a.x + __ldg(a.col + k));
       acc = warp_sum(acc);
-      if (lane == 0)
+      if (lane == 0 && MODE >= SPMV_CHEB_START)
+      {
+         RowOps o;
+         cheb_load<MODE>(a, r, o);
+         double yn = cheb_epilogue<MODE>(a, o, (MODE == SPMV_CHEB_START || MODE == SPMV_CHEB_ONE) ? __dadd_rn(o.b, -acc) : acc);
+         yn = store_out<MODE>(a, r, yn, o.d, 0.0);
+         if (DOT) dacc += a.dotv[r] * yn;
+      }
+      else if (lane == 0)
       {
          double yn;
          if (MODE == SPMV_SET || MODE == SPMV_SET_DIV || MODE == SPMV_GS_STEP) yn = acc;
@@ -771,6 +818,7 @@ int spmv_launch(const DevCSR &A, int mode, const SpmvArgs &s, const OffdFuse *of
    }
    d.exp = HaloExport();
    d.exp_y2 = s.export_y2 ? 1 : 0;
+   d.uo = s.uo;
    // Folding the export into this kernel saves the consumer's pack kernel (~13 us).  The exporting variants
    // compile to the same register budget as the non-exporting multi-rank ones (32 for SET / RESIDUAL /
    // ADD, 40 for the rest -- guarded by tests/test_abi_and_host.py), so every product folds; the tunable
@@ -788,8 +836,46 @@ int spmv_launch(const DevCSR &A, int mode, const SpmvArgs &s, const OffdFuse *of
       case SPMV_SET_DIV: return launch_mode<SPMV_SET_DIV>(A, d, dot);
       case SPMV_JACOBI2: return launch_mode<SPMV_JACOBI2>(A, d, dot);
       case SPMV_GS_STEP: return launch_mode<SPMV_GS_STEP>(A, d, dot);
+      case SPMV_CHEB_START: return launch_mode<SPMV_CHEB_START>(A, d, dot);
+      case SPMV_CHEB_STEP: return launch_mode<SPMV_CHEB_STEP>(A, d, dot);
+      case SPMV_CHEB_FIN: return launch_mode<SPMV_CHEB_FIN>(A, d, dot);
+      case SPMV_CHEB_ONE: return launch_mode<SPMV_CHEB_ONE>(A, d, dot);
    }
    return set_error(HDK_ERR_INVALID, "unknown spmv mode %d", mode);
+}
+
+// Chebyshev epilogue on a finished row result (levels whose off-rank part is added by a correction
+// kernel, and the zero-guess start where f - A 0 = f): the expressions of the fused kernels
+template <int MODE>
+__global__ void __launch_bounds__(ST) k_cheb_epi(SpmvDev a, const double *__restrict__ acc)
+{
+   for (int r = blockIdx.x * ST + threadIdx.x; r < a.nrows; r += gridDim.x * ST)
+   {
+      RowOps o;
+      o.yo = 0.0;
+      cheb_load<MODE>(a, r, o);
+      store_out<MODE>(a, r, cheb_epilogue<MODE>(a, o, acc[r]), o.d, 0.0);
+   }
+}
+
+int cheb_epilogue_pass(int mode, int n, const double *acc, const SpmvArgs &s)
+{
+   if (n <= 0) return HDK_OK;
+   SpmvDev d;
+   memset(&d, 0, sizeof(d));
+   d.b = s.b; d.d = s.d; d.y = s.y; d.y2 = s.y2; d.alpha = s.alpha; d.uo = s.uo; d.nrows = n;
+   int grid = cdiv(n, ST);
+   if (grid > g.sm_count * 8) grid = g.sm_count * 8;
+   switch (mode)
+   {
+      case SPMV_CHEB_START: k_cheb_epi<SPMV_CHEB_START><<<grid, ST, 0, g.stream>>>(d, acc); break;
+      case SPMV_CHEB_STEP: k_cheb_epi<SPMV_CHEB_STEP><<<grid, ST, 0, g.stream>>>(d, acc); break;
+      case SPMV_CHEB_FIN: k_cheb_epi<SPMV_CHEB_FIN><<<grid, ST, 0, g.stream>>>(d, acc); break;
+      case SPMV_CHEB_ONE: k_cheb_epi<SPMV_CHEB_ONE><<<grid, ST, 0, g.stream>>>(d, acc); break;
+      default: return set_error(HDK_ERR_INVALID, "unknown Chebyshev epilogue %d", mode);
+   }
+   HDK_LAUNCH_CHECK();
+   return HDK_OK;
 }
 
 // ---------------------------------------------------------------------------------------

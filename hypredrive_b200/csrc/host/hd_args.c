@@ -120,7 +120,11 @@ static const hd_field f_amg_rlx[] = {
    FM(hd_amg_args, down_type, map_relax), FM(hd_amg_args, up_type, map_relax), FM(hd_amg_args, coarse_type, map_coarse),
    FI(hd_amg_args, down_sweeps), FI(hd_amg_args, up_sweeps), FI(hd_amg_args, coarse_sweeps), FI(hd_amg_args, num_sweeps),
    FI(hd_amg_args, order), FM(hd_amg_args, points, map_points), FD(hd_amg_args, weight), FD(hd_amg_args, outer_weight),
-   FX("chebyshev"), FEND};
+   FEND};
+static const hd_field f_amg_cheby[] = {
+   {"order", F_INT, OFF(hd_amg_args, cheby_order), NULL, 0}, {"fraction", F_DBL, OFF(hd_amg_args, cheby_fraction), NULL, 0},
+   {"eig_est", F_INT, OFF(hd_amg_args, cheby_eig_est), NULL, 0}, {"variant", F_INT, OFF(hd_amg_args, cheby_variant), NULL, 0},
+   {"scale", F_INT, OFF(hd_amg_args, cheby_scale), NULL, 0}, FEND};
 static const hd_field f_amg_smt[] = {
    {"type", F_MAP, OFF(hd_amg_args, smooth_type), map_smooth, 0}, {"num_levels", F_INT, OFF(hd_amg_args, smooth_num_levels), NULL, 0},
    {"num_sweeps", F_INT, OFF(hd_amg_args, smooth_num_sweeps), NULL, 0}, FX("fsai"), FX("ilu"), FEND};
@@ -215,6 +219,7 @@ void hd_amg_defaults(hd_amg_args *a)
    a->relax_type = -1; a->down_type = 18; a->up_type = 18; a->coarse_type = 9;
    a->down_sweeps = -1; a->up_sweeps = -1; a->coarse_sweeps = 1; a->num_sweeps = 1; a->order = 0; a->points = 0;
    a->weight = 1.0; a->outer_weight = 1.0;
+   a->cheby_order = 2; a->cheby_fraction = 0.3; a->cheby_eig_est = 10; a->cheby_variant = 0; a->cheby_scale = 1;
    a->smooth_type = 5; a->smooth_num_levels = 0; a->smooth_num_sweeps = 1;
 }
 
@@ -256,7 +261,14 @@ static void parse_amg_block(hd_node *blk, hd_amg_args *a)
    if ((s = hd_yaml_find(blk, "interpolation"))) { s->used = 1; apply_fields(s, f_amg_int, a, "amg:interpolation", NULL); }
    if ((s = hd_yaml_find(blk, "coarsening"))) { s->used = 1; apply_fields(s, f_amg_csn, a, "amg:coarsening", NULL); }
    if ((s = hd_yaml_find(blk, "aggressive"))) { s->used = 1; apply_fields(s, f_amg_agg, a, "amg:aggressive", NULL); }
-   if ((s = hd_yaml_find(blk, "relaxation"))) { s->used = 1; apply_fields(s, f_amg_rlx, a, "amg:relaxation", NULL); }
+   if ((s = hd_yaml_find(blk, "relaxation")))
+   {
+      static const char *rlx_nested[] = {"chebyshev", NULL};
+      s->used = 1;
+      apply_fields(s, f_amg_rlx, a, "amg:relaxation", rlx_nested);
+      hd_node *c;
+      if ((c = hd_yaml_find(s, "chebyshev"))) { c->used = 1; apply_fields(c, f_amg_cheby, a, "amg:relaxation:chebyshev", NULL); }
+   }
    if ((s = hd_yaml_find(blk, "smoother"))) { s->used = 1; apply_fields(s, f_amg_smt, a, "amg:smoother", NULL); }
 }
 
@@ -615,6 +627,8 @@ void hd_amg_to_hdk(const hd_amg_args *a, hdk_amg_params *p)
    p->agg_num_levels = a->agg_num_levels; p->agg_num_paths = a->agg_num_paths;
    p->agg_interp_type = a->agg_prolongation_type; p->agg_max_nnz_row = a->agg_max_nnz_row;
    p->agg_trunc_factor = a->agg_trunc_factor;
+   p->cheby_order = a->cheby_order; p->cheby_fraction = a->cheby_fraction; p->cheby_eig_est = a->cheby_eig_est;
+   p->cheby_variant = a->cheby_variant; p->cheby_scale = a->cheby_scale;
 }
 
 /* systems AMG (num_functions > 1) runs hypre's unknown approach only: the nodal approach and
@@ -678,6 +692,46 @@ int hd_amg_check(const hd_amg_args *a)
       {
          hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
          hd_err_msg("amg:aggressive:num_levels = %d is not supported with num_functions = %d", a->agg_num_levels, a->num_functions);
+         bad = 1;
+      }
+   }
+   /* Chebyshev smoothing: the keys only matter when a phase relaxes with type 16 */
+   if (a->down_type == 16 || a->up_type == 16 || a->coarse_type == 16)
+   {
+      if (a->cheby_order < 1 || a->cheby_order > 4)
+      {
+         hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+         hd_err_msg("amg:relaxation:chebyshev:order must be in 1..4 (got %d)", a->cheby_order);
+         bad = 1;
+      }
+      if (!(a->cheby_fraction > 0.0 && a->cheby_fraction <= 1.0))
+      {
+         hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+         hd_err_msg("amg:relaxation:chebyshev:fraction must be in (0, 1] (got %g)", a->cheby_fraction);
+         bad = 1;
+      }
+      if (a->cheby_eig_est < 0)
+      {
+         hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+         hd_err_msg("amg:relaxation:chebyshev:eig_est must be at least 0 (got %d)", a->cheby_eig_est);
+         bad = 1;
+      }
+      if (a->cheby_variant == 1)
+      {
+         hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+         hd_err_msg("amg:relaxation:chebyshev:variant 1 is not supported: only variant 0 has a device implementation");
+         bad = 1;
+      }
+      else if (a->cheby_variant != 0)
+      {
+         hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+         hd_err_msg("amg:relaxation:chebyshev:variant must be 0 or 1 (got %d)", a->cheby_variant);
+         bad = 1;
+      }
+      if (a->cheby_scale != 0 && a->cheby_scale != 1)
+      {
+         hd_err_set(HYPREDRV_ERROR_INVALID_VAL);
+         hd_err_msg("amg:relaxation:chebyshev:scale must be 0 or 1 (got %d)", a->cheby_scale);
          bad = 1;
       }
    }

@@ -91,6 +91,9 @@ typedef struct
    /* relaxation */
    int    relax_type, down_type, up_type, coarse_type, down_sweeps, up_sweeps, coarse_sweeps, num_sweeps, order, points;
    double weight, outer_weight;
+   /* relaxation:chebyshev (hypre HYPRE_BoomerAMGSetCheby{Order,Fraction,EigEst,Variant,Scale}) */
+   int    cheby_order, cheby_eig_est, cheby_variant, cheby_scale;
+   double cheby_fraction;
    /* complex smoother */
    int    smooth_type, smooth_num_levels, smooth_num_sweeps;
 } hd_amg_args;

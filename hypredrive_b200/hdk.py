@@ -29,7 +29,9 @@ class AmgParams(C.Structure):
                 ("keep_transpose", C.c_int), ("print_level", C.c_int),
                 ("num_functions", C.c_int), ("dof_func", C.POINTER(C.c_int32)),
                 ("agg_num_levels", C.c_int), ("agg_num_paths", C.c_int), ("agg_interp_type", C.c_int),
-                ("agg_max_nnz_row", C.c_int), ("agg_trunc_factor", C.c_double)]
+                ("agg_max_nnz_row", C.c_int), ("agg_trunc_factor", C.c_double),
+                ("cheby_order", C.c_int), ("cheby_fraction", C.c_double), ("cheby_eig_est", C.c_int),
+                ("cheby_variant", C.c_int), ("cheby_scale", C.c_int)]
 
 
 class Krylov(C.Structure):
@@ -87,6 +89,7 @@ def lib():
         L.hdk_amg_get_measure.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.hdk_amg_get_dof_func.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.hdk_amg_get_l1.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
+        L.hdk_amg_get_cheby.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
         L.hdk_pcg.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Krylov)]
         L.hdk_gmres.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Krylov)]
         L.hdk_fgmres.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Krylov)]
@@ -308,6 +311,14 @@ class DAmg:
         out = np.empty(self.level_info(l)["rows"], dtype=np.float64)
         check(lib().hdk_amg_get_l1(self.h, l, out.ctypes.data))
         return out
+
+    def cheby(self, l):
+        """Chebyshev data of level l (relax 16): dict(eig=(max_eig, min_eig), coefs=c_0.., ds=D^{-1/2})."""
+        eig = np.empty(2, dtype=np.float64)
+        coefs = np.empty(4, dtype=np.float64)
+        ds = np.empty(self.level_info(l)["rows"], dtype=np.float64)
+        check(lib().hdk_amg_get_cheby(self.h, l, eig.ctypes.data, coefs.ctypes.data, ds.ctypes.data))
+        return dict(eig=(float(eig[0]), float(eig[1])), coefs=coefs[:self.params.cheby_order].copy(), ds=ds)
 
     def apply(self, r: DVec, z: DVec):
         check(lib().hdk_amg_apply(self.h, r.p, z.p))

@@ -126,7 +126,7 @@ typedef struct
    int    interp_type;     /* 6 = extended+i */
    int    max_nnz_row;     /* 4 */
    double trunc_factor;    /* 0 */
-   int    relax_down, relax_up, relax_coarse; /* 18 l1-Jacobi, 7 Jacobi, 11/12 two-stage GS, 9 GE */
+   int    relax_down, relax_up, relax_coarse; /* 18 l1-Jacobi, 7 Jacobi, 11/12 two-stage GS, 16 Chebyshev, 9 GE */
    int    sweeps_down, sweeps_up, sweeps_coarse;
    double relax_weight, outer_weight;
    int    rand_seed;       /* 2747 */
@@ -146,6 +146,15 @@ typedef struct
    int    agg_interp_type;  /* 4 = multipass */
    int    agg_max_nnz_row;  /* 0 */
    double agg_trunc_factor; /* 0 */
+   /* Chebyshev smoothing (relax 16, hypre HYPRE_BoomerAMGSetCheby*): per level, the eigenvalue bounds of
+    * C A (C = D^{-1}, D = diag|a_ii|, when scaled; C = I otherwise) from cheby_eig_est CG-Lanczos steps
+    * (0: Gershgorin bounds), the interval [lower, 1.1 max] with lower = min + fraction (1.1 max - min),
+    * and the monomial coefficients of the order-cheby_order polynomial; rule in DESIGN.md section 4 */
+   int    cheby_order;     /* 2: passes over A per sweep, 1..4 */
+   double cheby_fraction;  /* 0.3: (0, 1] */
+   int    cheby_eig_est;   /* 10: CG steps of the eigenvalue estimate, 0 = Gershgorin */
+   int    cheby_variant;   /* 0 (1 has no device implementation and is rejected) */
+   int    cheby_scale;     /* 1: smooth with D^{-1/2} A D^{-1/2}; 0: with A */
 } hdk_amg_params;
 
 void hdk_amg_default_params(hdk_amg_params *p);
@@ -177,6 +186,10 @@ int hdk_amg_get_cf(const hdk_amg *M, int level, int32_t *cf_h);
 int hdk_amg_get_dof_func(const hdk_amg *M, int level, int32_t *dof_h);
 int hdk_amg_get_measure(const hdk_amg *M, int level, double *measure_h);
 int hdk_amg_get_l1(const hdk_amg *M, int level, double *l1_h);
+/* Chebyshev data of level l (a level whose sweeps use relax 16): eig_h[0] = max_eig, eig_h[1] = min_eig,
+ * coefs_h[0..cheby_order) the polynomial coefficients c_0.., ds_h (may be NULL) this rank's D^{-1/2}
+ * (all ones when cheby_scale = 0) */
+int hdk_amg_get_cheby(const hdk_amg *M, int level, double *eig_h, double *coefs_h, double *ds_h);
 double hdk_amg_operator_complexity(const hdk_amg *M);
 /* algorithmic HBM bytes moved by one V-cycle (sum over levels, see DESIGN.md) */
 double hdk_amg_vcycle_bytes(const hdk_amg *M);
@@ -217,7 +230,8 @@ int hdk_bicgstab(const hdk_csr *A, hdk_amg *M, const double *b_d, double *x_d, h
  * one hot kernel on the compute stream, CUDA-event timed (bench.py roofline leg).
  * kernel: 0 = SpMV y=Ax, 1 = l1-Jacobi sweep fused with residual, 2 = residual r=b-Ax,
  *         3 = PCG fused x/r update + <r,r> + first V-cycle sweep (the 64 B/row variant the solve runs),
- *         4 = V-cycle, 5 = PCG p = z + beta p, 6 = one fused two-stage Gauss-Seidel sweep (relax 11/12) */
+ *         4 = V-cycle, 5 = PCG p = z + beta p, 6 = one fused two-stage Gauss-Seidel sweep (relax 11/12),
+ *         9 = one Chebyshev sweep (relax 16) on the fine level of M */
 int hdk_time_kernel(const hdk_csr *A, hdk_amg *M, int kernel, int reps, double *avg_ms,
                     double *algorithmic_bytes);
 /* number of kernel launches issued by this library since the last call (and reset) */
